@@ -4,7 +4,7 @@
 Metric (BASELINE.json): Gibbs sweeps/sec + Vecchia log-lik evals/sec at n = 1M, m = 10.  One STEP = one full chromatic
 Gibbs sweep of the latent field (all colour classes, Philox normals) + one Vecchia log-likelihood evaluation.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N = 1: config 3 (synthetic U(0,1)^2 sites, n = 1 000 000, m = 10, exponential_isotropic, range 0.05, sigma^2 = 1, tau^2 = 0.1).
   `value` = steps/s, inputs resident in HBM, CUDA events on the library's stream; `e2e` = the same step through the C ABI with
@@ -158,6 +158,21 @@ def build_problem(n, m, seed, reordering="random"):
     return rng, locs, nn, coloring, locs_match, t
 
 
+DUMP_MAX_FIELD = 4_000_000   # float64 values (32 MB): a larger field is dumped as a fixed, seeded sample of this many sites
+
+
+def dump_outputs(out_dir, field, loglik):
+    """--dump-outputs: what the last timed step returns to a caller, the swept field and its Vecchia log-lik, as float64 .npy files,
+    so that two builds run with the same arguments can be compared output for output"""
+    os.makedirs(out_dir, exist_ok=True)
+    if field.size > DUMP_MAX_FIELD:
+        idx = np.sort(np.random.default_rng(0).choice(field.size, DUMP_MAX_FIELD, replace=False))
+        np.save(os.path.join(out_dir, "field_sample.npy"), field[idx])
+    else:
+        np.save(os.path.join(out_dir, "field.npy"), field)
+    np.save(os.path.join(out_dir, "loglik.npy"), np.array([loglik], dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # reference arm / cpu_baseline: the oracle restatement of the reference's CPU path (R + GpGp + Matrix are not in this image)
 # ---------------------------------------------------------------------------------------------------------------------
@@ -279,6 +294,8 @@ def run_single(a):
     launches = nb.launch_count() - launches0
     total_ms = float(ms_steps.sum())
     value = a.steps / (total_ms * 1e-3)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, ctx.field_get(), ctx.loglik(0.0, ls))   # nngp_time_op's step takes its log-lik at beta_0 = 0
     # component timings (same stream, same events; >= 50 repetitions, median and min -- SURVEY.md 8d)
     reps = max(50, min(a.steps, 200))
     comp = {}
@@ -717,14 +734,20 @@ def main():
     ap.add_argument("--mode", default="auto", choices=["auto", "single", "sharded"])
     ap.add_argument("--transport", default="p2p", choices=["p2p", "nccl"], help="sharded mode: halo transport")
     ap.add_argument("--range", dest="range_", type=float, default=None, help="covariance range (default 0.05; BASELINE config 4 is run with 0.02)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="single GPU: write the field and log-lik of the last timed step as DIR/field.npy (DIR/field_sample.npy, a seeded "
+                         f"sample of {DUMP_MAX_FIELD} sites, above that size) and DIR/loglik.npy, float64")
     a = ap.parse_args()
     if a.range_ is not None:
         global RANGE
         RANGE = a.range_
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    sharded = a.mode == "sharded" or (a.mode == "auto" and world > 1)
+    if a.dump_outputs and (a.impl == "reference" or sharded):
+        ap.error("--dump-outputs is implemented for the single-GPU run of the library (--impl ours, one rank)")
     if a.impl == "reference":
         run_reference(a)
-    elif a.mode == "sharded" or (a.mode == "auto" and world > 1):
+    elif sharded:
         run_sharded(a)
     else:
         run_single(a)

@@ -40,3 +40,9 @@ def test_product_arm_fails_loudly_without_a_gpu():
     r = run_bench("--steps", "1", "--warmup", "1", "--n", "2000")
     assert r.returncode != 0
     assert "no CPU fallback" in (r.stderr + r.stdout)
+
+
+def test_dump_outputs_is_refused_where_it_is_not_implemented(tmp_path):
+    r = run_bench("--impl", "reference", "--n", "2000", "--steps", "1", "--dump-outputs", str(tmp_path))
+    assert r.returncode != 0 and "--dump-outputs" in r.stderr
+    assert list(tmp_path.iterdir()) == []

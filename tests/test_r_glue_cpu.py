@@ -3,7 +3,7 @@ every .C("nngp_...") call names an exported ABI function and passes exactly as m
 include/nngp_b200.h has parameters, named and ordered like them, with `status` last (.C() matches by position: a wrong
 count or order corrupts memory at run time in R), and of the right KIND: .C() hands a double vector over as double *, an integer
 vector as int *, and a character vector as char ** (never char *).  The patch for mcmc_nngp_initialize.R must apply to the
-reference's file, and the .Call glue must compile against the R API declarations it uses."""
+reference's lines it changes (tests/golden/mcmc_nngp_initialize_excerpt.R), and the .Call glue must compile against the R API declarations it uses."""
 import os
 import re
 import shutil
@@ -142,9 +142,7 @@ def test_initialize_patch_applies_to_the_reference_and_calls_only_bound_wrappers
     assert used >= {"nngp_find_ordered_nn", "nngp_greedy_coloring", "nngp_chain_context", "nngp_factor_build", "nngp_field_init", "nngp_field_get"}
     for f in used:
         assert re.search(rf"^{f}\s*=\s*function", glue, flags=re.M), f      # every wrapper the patch calls exists in R/nngp_b200.R
-    ref = "/root/reference/Scripts/mcmc_nngp_initialize.R"
-    if not os.path.exists(ref) or not shutil.which("patch"):
-        return                                                                # the reference tree is not on the GPU box
+    ref = os.path.join(ROOT, "tests", "golden", "mcmc_nngp_initialize_excerpt.R")   # the reference's lines the patch touches
     import tempfile
     with tempfile.TemporaryDirectory() as d:
         os.makedirs(os.path.join(d, "Scripts"))
