@@ -1,6 +1,10 @@
 """Seeded synthetic NNGP problems shared by the parity tests, smoke() and bench.py."""
 from __future__ import annotations
 
+import json
+import os
+from decimal import Decimal, localcontext
+
 import numpy as np
 
 import nngp_b200 as nb
@@ -55,3 +59,105 @@ def make_regression_problem(n, m, seed=0, n_extra_obs=0, p_locs=2, p_obs=1, rang
     P.update(X=X, xlocs=np.arange(1, p_locs + 1, dtype=np.int32), first_obs=(first + 1).astype(np.int32), solve_1XT1X=S,
              chol_solve_1XT1X=np.linalg.cholesky(S).T, beta_true=beta_true, y=y, w=w)
     return P
+
+
+# ---------------------------------------------------------------------------------------------------------------------------
+# Kernel probes: a problem whose probe rows decouple into exact 2 x 2 blocks, so that the kernel value the factor build used for
+# one distance can be read off a factor row.  Anchor A (site 1) sits at the origin; anchors 2..m sit 1e4 apart on the negative
+# first axis, so that every kernel value between them, or between them and a probe, is exactly 0 in double; probe row i is the
+# site (x_i, 0[, 0, 0]) and lists A in slot 1 and the far anchors in slots 2..m (a full row: the specialised kernels take it).
+# With covparms (s2, 1, [nu,] tau) the block of a probe row is s2 [[1 + tau, rho], [rho, 1 + tau]] plus an identity-scaled
+# diagonal part for the far anchors, hence
+#     rho(x) = -Linv[i, 1] / Linv[i, 0] * (1 + tau),      Linv[i, 0]^-2 = s2 ((1 + tau) - rho^2 / (1 + tau)).
+# ---------------------------------------------------------------------------------------------------------------------------
+PROBE_REFERENCE = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "kernel_probe_reference.json")
+
+
+def make_probe_problem(m, d, xs):
+    """Probe rows m+1 .. m+len(xs) at (x, 0, ...); all-zero colouring (a context without sweeps), no observations."""
+    xs = np.asarray(xs, dtype=np.float64)
+    n = m + xs.size
+    locs = np.zeros((n, d))
+    locs[1:m, 0] = -1e4 * np.arange(1, m)
+    locs[m:, 0] = xs
+    nn = np.full((n, m + 1), nb.NA_INT, dtype=np.int32)
+    nn[:, 0] = np.arange(1, n + 1)
+    for k in range(1, m):                       # anchor rows: partial, every earlier anchor
+        nn[k, 1:k + 1] = np.arange(1, k + 1)
+    nn[m:, 1:] = np.arange(1, m + 1)
+    return dict(locs=locs, NNarray=nn, coloring=np.zeros(n, dtype=np.int32), locs_match=np.zeros(0, dtype=np.int32), n=n, m=m, d=d)
+
+
+def probe_covparms(nu, s2, tau):
+    """isotropic covparms with range 1 (the scaled distance is x): exponential when nu is None"""
+    return [s2, 1.0, tau] if nu is None else [s2, 1.0, nu, tau]
+
+
+def load_probe_reference(path=PROBE_REFERENCE):
+    """x (exact doubles) and, per family, the 50-digit rho split into a double and its remainder, and kappa = |x dlog(rho)/dx|"""
+    with open(path) as f:
+        ref = json.load(f)
+    ref["x"] = np.array([float.fromhex(h) for h in ref["x"]])
+    with localcontext() as ctx:
+        ctx.prec = 80
+        for fam in ref["families"]:
+            hi = [float(r) for r in fam["rho"]]
+            fam["rho_hi"] = np.array(hi)
+            fam["rho_lo"] = np.array([float(Decimal(r) - Decimal(h)) for r, h in zip(fam["rho"], hi)])
+            fam["kappa"] = np.array([float(k) for k in fam["kappa"]])
+    return ref
+
+
+# regimes of the device's Matern evaluation by the squared scaled distance s (kernels.cuh: MT_EMIN, MTS_E0, MT_ESCALED, MTS_E1,
+# MT_EMAX); the specialised kernels read [2^-26, 2^6) from shared memory, the generic ones from the global table
+PROBE_REGIMES = [(0.0, "s = 0"), (2.0 ** -1074, "exact K_nu, s < 2^-80"), (2.0 ** -80, "global table, [2^-80, 2^-26)"),
+                 (2.0 ** -26, "smem table, [2^-26, 4)"), (4.0, "smem table e^x-scaled, [4, 2^6)"),
+                 (2.0 ** 6, "global table e^x-scaled, [2^6, 2^20)"), (2.0 ** 20, "exact K_nu, s >= 2^20")]
+
+
+def probe_regime(x):
+    s = x * x
+    return [name for lo, name in PROBE_REGIMES if s >= lo][-1]
+
+
+def probe_errors(Linv, m, fam, s2, tau):
+    """Per probe row: (relative error of rho, its bound, |conditional variance error|, its bound); NaN where not checked.
+    rho >= 1e-280: relative to the 50-digit value, bound 1e-13 + kappa 2^-52 (kappa: the conditioning of rho in its argument, the
+    rounding of s = x^2 and of sqrt(s) alone moves rho by kappa ulps).  Smaller rho: absolute 1e-280.  With tau = 0, probes where
+    1 - rho^2 < 1e-10 are skipped (a singular block).  The conditional variance Linv[i, 0]^-2 is compared with
+    s2 ((1 + tau) - rho_row^2 / (1 + tau)) for the rho read off the same row (checked above): this isolates the pivot arithmetic,
+    whose bound is 8 ulps of s2 (1 + tau)."""
+    L = Linv[m:]
+    rho_hi, rho_lo, kappa = fam["rho_hi"], fam["rho_lo"], fam["kappa"]
+    with np.errstate(invalid="ignore", divide="ignore"):      # tau = 0, x = 0: singular block (skipped below)
+        got = -L[:, 1] / L[:, 0] * (1.0 + tau)
+        var = 1.0 / L[:, 0] ** 2
+    err = np.abs((got - rho_hi) - rho_lo)
+    big = rho_hi >= 1e-280
+    rel = np.where(big, err / np.where(big, rho_hi, 1.0), err)
+    bound = np.where(big, 1e-13 + kappa * 2.0 ** -52, 1e-280)
+    var_err = np.abs(var - s2 * ((1.0 + tau) - got ** 2 / (1.0 + tau)))
+    var_bound = np.full(got.shape, 8 * np.spacing(s2 * (1.0 + tau)))
+    if tau == 0.0:
+        skip = 1.0 - rho_hi ** 2 < 1e-10
+        rel[skip] = np.nan
+        var_err[skip] = np.nan
+    return rel, bound, var_err, var_bound
+
+
+def probe_failures(Linv, m, ref, fam, s2, tau, label, worst=None, skip=None):
+    """Messages for the probes over their bounds (regime, nu, x, the kernel instantiation); `worst` collects the largest relative
+    error of rho per regime (Matern) or for the exponential family when given; probes where `skip` is true are not checked."""
+    rel, bound, var_err, var_bound = probe_errors(Linv, m, fam, s2, tau)
+    out = []
+    for i, x in enumerate(ref["x"]):
+        if skip is not None and skip[i]:
+            continue
+        reg = probe_regime(x)
+        if worst is not None and np.isfinite(rel[i]) and fam["rho_hi"][i] >= 1e-280:
+            key = reg if fam["nu"] is not None else "exponential"
+            worst[key] = max(worst.get(key, 0.0), float(rel[i]))
+        if not (rel[i] <= bound[i] or np.isnan(rel[i])) or not (var_err[i] <= var_bound[i] or np.isnan(var_err[i])):
+            out.append(f"{label} {fam['covfun']} nu={fam['nu']!r} s2={s2} tau={tau} x={x!r} [{reg}]: rho rel err {rel[i]:.3g} "
+                       f"(bound {bound[i]:.3g}), cond. variance err {var_err[i]:.3g} (bound {var_bound[i]:.3g})")
+    return out

@@ -35,6 +35,29 @@ CASES = [
     ("matern_isotropic", 2, 20, [1.0, 0.1, 0.6, 0.0]),
     ("matern_scaledim", 2, 5, [1.0, 0.05, 0.11, 0.9, 0.0]),
     ("matern_spacetime", 3, 5, [1.0, 0.2, 0.5, 0.55, 0.0]),
+    # generic<16> (M = 9..16), generic<24> (M = 17..24, and m = 20 at d = 3), generic<32> (M = 25..32); the row kernels at MT = 0
+    ("exponential_isotropic", 2, 8, [1.0, 0.1, 0.0]),
+    ("matern_isotropic", 3, 12, [1.0, 0.25, 0.8, 0.0]),
+    ("exponential_spacetime", 3, 15, [1.0, 0.2, 0.4, 0.0]),
+    ("matern_isotropic", 2, 16, [1.0, 0.02, 1.2, 0.0]),     # range 0.05: conditioning alone puts precision_diag at 1.4e-10
+    ("exponential_isotropic", 3, 20, [1.0, 0.3, 0.0]),
+    ("matern_scaledim", 2, 21, [1.0, 0.05, 0.08, 0.6, 0.0]),
+    ("exponential_isotropic", 2, 24, [1.0, 0.1, 0.0]),
+    ("matern_isotropic", 3, 24, [1.0, 0.25, 0.9, 0.0]),
+    ("exponential_scaledim", 3, 31, [1.0, 0.2, 0.3, 0.25, 0.0]),
+    ("matern_isotropic", 2, 31, [1.0, 0.05, 0.7, 0.0]),
+    # d = 1 and d = 4 (transformed dimensions 1 and 4: generic kernels only)
+    ("exponential_isotropic", 1, 10, [1.0, 0.001, 0.0]),
+    ("matern_isotropic", 1, 5, [1.0, 0.001, 0.4, 0.0]),
+    ("exponential_isotropic", 4, 10, [1.0, 0.4, 0.0]),
+    ("exponential_scaledim", 4, 10, [1.0, 0.3, 0.4, 0.5, 0.6, 0.0]),
+    ("matern_spacetime", 4, 10, [1.0, 0.4, 0.5, 0.85, 0.0]),
+    ("matern_scaledim", 4, 20, [1.0, 0.5, 0.4, 0.6, 0.3, 0.45, 0.0]),
+    # a nugget (diagonal s2 (1 + tau)) and variances other than 1 (the Matern table carries the variance in its coefficients)
+    ("matern_isotropic", 2, 10, [1.0, 0.07, 0.75, 0.3]),
+    ("exponential_isotropic", 2, 10, [0.4, 0.07, 0.2]),
+    ("matern_isotropic", 2, 20, [2.5, 0.1, 0.6, 0.0]),
+    ("matern_isotropic", 3, 5, [3.7, 0.3, 1.45, 0.1]),
 ]
 
 
@@ -64,14 +87,48 @@ def test_factor_and_products(covfun, d, m, cp, layout):
 
 
 def test_sphere_factor():
+    """*_sphere: transformed dimension 3 -- reg<6,3>, reg<11,3>, and at m = 20 generic<24> (thread per row) or warp<21,3>"""
     rng = np.random.default_rng(3)
-    n, m = 3000, 5
+    n = 3000
     lonlat = np.column_stack([rng.uniform(-120, -70, n), rng.uniform(25, 50, n)])
-    P = make_problem(n, m, locs=lonlat, seed=3)
-    for covfun, cp in (("exponential_sphere", [1.0, 0.05, 0.0]), ("matern_sphere", [1.0, 0.05, 0.8, 0.0])):
-        with nb.NNGPContext(lonlat, P["NNarray"], P["coloring"], P["locs_match"], covfun) as ctx:
-            assert ctx.factor_build(cp) == 0
-            assert rel_rows(ctx.factor_get(), O.vecchia_Linv(cp, covfun, lonlat, P["NNarray"])) < 1e-9
+    for m in (5, 10, 20):
+        P = make_problem(n, m, locs=lonlat, seed=3)
+        for covfun, cp in (("exponential_sphere", [1.0, 0.05, 0.0]), ("matern_sphere", [1.0, 0.05, 0.8, 0.0])):
+            Lo = O.vecchia_Linv(cp, covfun, lonlat, P["NNarray"])
+            with nb.NNGPContext(lonlat, P["NNarray"], P["coloring"], P["locs_match"], covfun) as ctx:
+                for fv in ((0, 1) if m == 20 else (0,)):
+                    ctx.set_option("factor_variant", fv)
+                    assert ctx.factor_build(cp) == 0, (m, covfun, fv)
+                    assert rel_rows(ctx.factor_get(), Lo) < 1e-9, (m, covfun, fv)
+
+
+@pytest.mark.parametrize("n", [4001, 20000])
+@pytest.mark.parametrize("covfun,d,cp", [("exponential_isotropic", 2, [1.0, 0.1, 0.0]), ("exponential_spacetime", 3, [1.0, 0.2, 0.4, 0.0]),
+                                         ("matern_isotropic", 2, [1.0, 0.1, 0.6, 0.0]), ("matern_isotropic", 3, [1.3, 0.25, 1.1, 0.2])])
+def test_warp_per_row_factor_build(n, covfun, d, cp):
+    """factor_variant = 1 (vecchia_factor_warp_kernel<21, dt>, m = 20) against the oracle: the first m (partial) rows go through
+    factor_row_generic on lane 0; n = 4001 ends in a ragged 32-row round and n = 20000 makes the grid-stride loop run more than one
+    round per block (the grid is min(ceil(n / 32), 2 n_SM) blocks); both slots; the triangular solve reads the level-ordered copy of
+    the factor that this kernel writes itself; a negative variance fails every pivot."""
+    m = 20
+    P = make_problem(n, m, d=d, seed=n + d)
+    cp2 = [cp[0] * 0.8, cp[1] * 1.3] + cp[2:]
+    Lo = O.vecchia_Linv(cp, covfun, P["locs"], P["NNarray"])
+    Lo2 = O.vecchia_Linv(cp2, covfun, P["locs"], P["NNarray"])
+    v = P["rng"].standard_normal(n)
+    with nb.NNGPContext(P["locs"], P["NNarray"], P["coloring"], P["locs_match"], covfun) as ctx:
+        ctx.set_option("factor_variant", 1)
+        assert ctx.factor_build(cp) == 0
+        assert ctx.factor_build(cp2, slot=nb.SLOT_PROPOSAL) == 0
+        Lg, Lg2 = ctx.factor_get(), ctx.factor_get(nb.SLOT_PROPOSAL)
+        assert rel_rows(Lg, Lo) < TOL and rel_rows(Lg2, Lo2) < TOL
+        assert rel_rows(Lg[:m], Lo[:m]) < TOL and np.all(Lg[P["NNarray"] == nb.NA_INT] == 0.0)
+        assert rel_vec(ctx.sptrsv(v), O.sparse_chol_solve(Lo, P["NNarray"], v)) < 1e-9
+        assert rel_vec(ctx.sptrsv(v, slot=nb.SLOT_PROPOSAL), O.sparse_chol_solve(Lo2, P["NNarray"], v)) < 1e-9
+        ctx.field_set(P["field"])
+        ll_o = O.ll_compressed_sparse_chol(Lo, P["field"] - 0.3, P["NNarray"], 0.4)
+        assert abs(ctx.loglik(0.3, 0.4) - ll_o) < TOL * abs(ll_o)
+        assert ctx.factor_build([-cp[0]] + cp[1:]) == n
 
 
 @pytest.mark.parametrize("n,m", [(1, 3), (5, 10), (12, 10), (40, 1), (1000, 10)])
@@ -92,25 +149,38 @@ def test_small_and_ragged(n, m):
 
 def test_not_positive_definite_is_flagged_not_fatal():
     """A block that fails the Cholesky pivot test (pivot <= 0 or NaN, LAPACK's criterion) is counted, not fatal: the caller
-    rejects the proposal (SURVEY.md 8b error convention)."""
-    P = make_problem(500, 5, seed=5)
-    with nb.NNGPContext(P["locs"], P["NNarray"], P["coloring"], P["locs_match"]) as ctx:
-        assert ctx.factor_build([-1.0, 0.2, 0.0]) == 500          # negative variance: every pivot fails
-        assert ctx.factor_build([1.0, 0.2, 0.0]) == 0             # and the context is still usable
-        _, bad = O.vecchia_Linv([-1.0, 0.2, 0.0], "exponential_isotropic", P["locs"], P["NNarray"], return_bad=True)
-        assert bad == 500
-    locs = P["locs"].copy()
-    locs[300] = locs[P["NNarray"][300, 1] - 1]          # exact duplicate of a neighbour: pivot is 0 up to rounding
-    with nb.NNGPContext(locs, P["NNarray"], P["coloring"], P["locs_match"]) as ctx:
-        assert ctx.factor_build([1.0, 0.2, 0.0]) in (0, 1)   # flagged or a huge-but-finite row, never a crash
+    rejects the proposal (SURVEY.md 8b error convention).  Every kernel family: reg<6,2>, generic<16>, reg<21,2,MINB=1>, warp<21,2>,
+    generic<32>, and d = 4."""
+    for m, d, fv in ((5, 2, 0), (12, 2, 0), (20, 2, 0), (20, 2, 1), (31, 2, 0), (10, 4, 0)):
+        case = dict(m=m, d=d, factor_variant=fv)
+        P = make_problem(500, m, d=d, seed=5)
+        with nb.NNGPContext(P["locs"], P["NNarray"], P["coloring"], P["locs_match"]) as ctx:
+            ctx.set_option("factor_variant", fv)
+            assert ctx.factor_build([-1.0, 0.2, 0.0]) == 500, case          # negative variance: every pivot fails
+            assert ctx.factor_build([1.0, 0.2, 0.0]) == 0, case             # and the context is still usable
+            _, bad = O.vecchia_Linv([-1.0, 0.2, 0.0], "exponential_isotropic", P["locs"], P["NNarray"], return_bad=True)
+            assert bad == 500
+        locs = P["locs"].copy()
+        twin = P["NNarray"][300, 1]
+        locs[300] = locs[twin - 1]                          # exact duplicate of a neighbour: pivot is 0 up to rounding
+        # every row whose block holds both copies is singular: each is flagged or a huge-but-finite row, never a crash
+        # (m = 5: 2 such rows); every other row is the oracle's
+        singular = np.any(P["NNarray"] == 301, axis=1) & np.any(P["NNarray"] == twin, axis=1)
+        with nb.NNGPContext(locs, P["NNarray"], P["coloring"], P["locs_match"]) as ctx:
+            ctx.set_option("factor_variant", fv)
+            assert 0 <= ctx.factor_build([1.0, 0.2, 0.0]) <= int(singular.sum()), case
+            Lo = O.vecchia_Linv([1.0, 0.2, 0.0], "exponential_isotropic", locs, P["NNarray"])
+            assert rel_rows(ctx.factor_get()[~singular], Lo[~singular]) < TOL, case
 
 
 @pytest.mark.parametrize("layout", [nb.LAYOUT_COLOR, nb.LAYOUT_COLOR_MORTON, nb.LAYOUT_MORTON])
-@pytest.mark.parametrize("m,n_extra,drop", [(10, 0, 0.0), (5, 300, 0.0), (10, 200, 0.3)])
+@pytest.mark.parametrize("m,n_extra,drop", [(10, 0, 0.0), (5, 300, 0.0), (10, 200, 0.3), (31, 100, 0.0), (12, 0, 0.2)])
 def test_chromatic_sweep_supplied_normals(layout, m, n_extra, drop):
-    """Same normals in the reference's hand-out order => same field as update_Gaussian.R:257-275 written literally."""
-    P = make_problem(3000, m, seed=21, n_extra_obs=n_extra, drop_obs_frac=drop)
-    cp = [1.0, 0.08, 0.0]
+    """Same normals in the reference's hand-out order => same field as update_Gaussian.R:257-275 written literally; generic neighbour
+    counts included (m = 31 at d = 2, m = 12 at d = 4)."""
+    d = 4 if m == 12 else 2
+    P = make_problem(3000, m, d=d, seed=21, n_extra_obs=n_extra, drop_obs_frac=drop)
+    cp = [1.0, 0.08 if d == 2 else 0.3, 0.0]
     beta_0, ls, lnv = 0.3, 0.2, -1.1
     Lo = O.vecchia_Linv(cp, "exponential_isotropic", P["locs"], P["NNarray"])
     pd = O.precision_diag(Lo, P["NNarray"])
@@ -196,22 +266,30 @@ def test_ancillary_beta0_and_field_init():
 
 
 def test_predict_sample():
-    n, n_pred, m = 1500, 700, 10
+    """predict.R:43-53 on the device: exponential and Matern with nu <= 1/2 (reachable through predict.R:37's 1.5 plogis) and near
+    3/2 at a generic neighbour count, every storage layout, new sites after the observed ones, every site new, and none new"""
+    n, n_pred = 1500, 700
     rng = np.random.default_rng(8)
     locs = rng.random((n + n_pred, 2))
-    nn = nb.find_ordered_nn(locs, m)
-    cp = [1.0, 0.2, 0.0]
-    Lo = O.vecchia_Linv(cp, "exponential_isotropic", locs, nn)
-    field = 0.3 + rng.standard_normal(n)
-    z = rng.standard_normal(n_pred)
-    want = O.predict_field_sample(Lo, nn, n, field, 0.3, 0.5, z)
-    with nb.NNGPContext(locs, nn, np.zeros(n + n_pred, dtype=np.int32), np.zeros(0, dtype=np.int32)) as ctx:   # all-zero colouring = no sweeps
-        ctx.factor_build(cp)
-        got = ctx.predict_sample(n, field, 0.3, 0.5, z)
-        with pytest.raises(nb.NNGPError) as e:                  # a context without a colouring refuses to sweep
-            ctx.gibbs_sweep(0.0, 0.0, 0.0, n_sweeps=1, seed=1)
-        assert e.value.status == 4
-    assert rel_vec(got, want) < 1e-9
+    field = 0.3 + rng.standard_normal(n + n_pred)
+    z = rng.standard_normal(n + n_pred)
+    for covfun, m, cp in (("exponential_isotropic", 10, [1.0, 0.2, 0.0]), ("matern_isotropic", 10, [1.0, 0.1, 0.3, 0.0]),
+                          ("matern_isotropic", 15, [1.0, 0.1, 1.45, 0.0])):
+        nn = nb.find_ordered_nn(locs, m)
+        Lo = O.vecchia_Linv(cp, covfun, locs, nn)
+        for layout in (nb.LAYOUT_COLOR, nb.LAYOUT_COLOR_MORTON, nb.LAYOUT_MORTON):
+            with nb.NNGPContext(locs, nn, np.zeros(n + n_pred, dtype=np.int32), np.zeros(0, dtype=np.int32), covfun, layout=layout) as ctx:   # all-zero colouring = no sweeps
+                assert ctx.factor_build(cp) == 0
+                for n0 in (n, 0, n + n_pred):
+                    case = dict(covfun=covfun, m=m, layout=layout, n_obs_sites=n0)
+                    got = ctx.predict_sample(n0, field[:n0], 0.3, 0.5, z[:n + n_pred - n0])
+                    want = O.predict_field_sample(Lo, nn, n0, field[:n0], 0.3, 0.5, z[:n + n_pred - n0])
+                    assert got.shape == (n + n_pred - n0,), case
+                    if n0 < n + n_pred:
+                        assert rel_vec(got, want) < 1e-9, case
+                with pytest.raises(nb.NNGPError) as e:                  # a context without a colouring refuses to sweep
+                    ctx.gibbs_sweep(0.0, 0.0, 0.0, n_sweeps=1, seed=1)
+                assert e.value.status == 4
 
 
 @pytest.mark.parametrize("covfun,shape", [("exponential_isotropic", [np.log(0.1)]), ("matern_isotropic", [np.log(0.1), 0.3])])
@@ -323,11 +401,12 @@ def test_error_paths():
     assert "not proper" in str(e.value)
 
 
-@pytest.mark.parametrize("variant", [0, 1, 2, 3])
+@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4])
 @pytest.mark.parametrize("n,m", [(20000, 10), (3000, 5)])
 def test_every_sweep_variant_matches_the_reference_loop(variant, n, m):
-    """All kernel variants of the sweep (PDL chain of tiles with and without the 6-CTAs/SM build, plain tiled launches, thread-per-site)
-    are the same map given the same normals; multi-sweep launches included (n = 20000 gives several CTAs per colour)."""
+    """All kernel variants of the sweep (PDL chain of tiles with and without the 6-CTAs/SM build, dependents triggered after the wait,
+    plain tiled launches, thread-per-site) are the same map given the same normals; multi-sweep launches included (n = 20000 gives
+    several CTAs per colour); the captured graph's replay and direct launches give the same field bit for bit."""
     P = make_problem(n, m, seed=77, n_extra_obs=n // 20)
     cp = [1.0, 0.05, 0.0]
     beta_0, ls, lnv = -0.2, 0.3, -0.9
@@ -348,11 +427,16 @@ def test_every_sweep_variant_matches_the_reference_loop(variant, n, m):
         ctx.field_set(P["field"])
         ctx.obs_set(P["y"])
         ctx.gibbs_sweep(beta_0, ls, lnv, n_sweeps=n_sweeps, z=z)
-        assert rel_vec(ctx.field_get(), f) < TOL
+        fz = ctx.field_get()
+        assert rel_vec(fz, f) < TOL
         # Philox draws are keyed by (seed, sweep counter, site): identical across variants
         ctx.field_set(P["field"])
         ctx.gibbs_sweep(beta_0, ls, lnv, n_sweeps=2, seed=5)
         a = ctx.field_get()
+        ctx.set_option("use_graph", 0)
+        ctx.field_set(P["field"])
+        ctx.gibbs_sweep(beta_0, ls, lnv, n_sweeps=n_sweeps, z=z)
+        assert np.array_equal(ctx.field_get(), fz)
     with nb.NNGPContext(P["locs"], P["NNarray"], P["coloring"], P["locs_match"], layout=nb.LAYOUT_COLOR) as ctx:
         ctx.set_option("sweep_variant", 3)
         ctx.factor_build(cp)
@@ -382,8 +466,15 @@ def test_both_solve_variants(solve_variant, level_copy, m):
         assert rel_vec(ctx.sptrsv(v), O.sparse_chol_solve(Lo, P["NNarray"], v)) < 1e-9
         assert rel_vec(ctx.sptrsv(v, slot=nb.SLOT_PROPOSAL), O.sparse_chol_solve(Lo2, P["NNarray"], v)) < 1e-9
         ctx.factor_accept()                                    # the proposal becomes the current factor: the copies swap with it
-        assert rel_vec(ctx.sptrsv(v), O.sparse_chol_solve(Lo2, P["NNarray"], v)) < 1e-9
+        x0 = ctx.sptrsv(v)
+        assert rel_vec(x0, O.sparse_chol_solve(Lo2, P["NNarray"], v)) < 1e-9
         assert rel_vec(ctx.sptrsv(v, slot=nb.SLOT_PROPOSAL), O.sparse_chol_solve(Lo, P["NNarray"], v)) < 1e-9
+        # the schedule knobs change which CTA takes which rows and when, never the arithmetic of a row (fixed association): the
+        # same solution bit for bit -- one CTA walking the whole DAG, 8 CTAs per SM, a back-off between polls, no graph replay
+        for opt, val, default in (("solve_window_ctas", 1, 0), ("solve_ctas_per_sm", 8, 1), ("solve_sleep_ns", 200, 0), ("use_graph", 0, 1)):
+            ctx.set_option(opt, val)
+            assert np.array_equal(ctx.sptrsv(v), x0), (opt, val)
+            ctx.set_option(opt, default)
 
 
 @pytest.mark.parametrize("commit_variant", [0, 1])
