@@ -64,7 +64,8 @@ class NNGPContext:
         L.check(st)
 
     OPTIONS = {"sweep_variant": 1, "solve_variant": 2, "use_graph": 3, "solve_ctas_per_sm": 4, "solve_sleep_ns": 5, "solve_level_copy": 6,
-               "solve_window_ctas": 7, "commit_variant": 8, "matern_table": 9, "loglik_variant": 10, "shard_ghost_ctas": 11, "shard_ghost_first": 12, "factor_variant": 14}
+               "solve_window_ctas": 7, "commit_variant": 8, "matern_table": 9, "loglik_variant": 10, "shard_ghost_ctas": 11, "shard_ghost_first": 12, "factor_variant": 14,
+               "loglik_from_residual": 15}
 
     def set_option(self, name: str, value: int):
         self._call("nngp_ctx_set_option", L.ci(self.OPTIONS[name]), L.ci(value))

@@ -225,6 +225,9 @@ struct Ctx {
     // SLOWER (44.7 vs 37.3 us at n = 1M, 128 vs 100 us at 4M, 96 vs 55 us at m = 20): the pass is bound by the latency of
     // the 8-byte field gathers, which wants 2048 resident threads per SM; a 100 KB ring leaves room for 512.
     int loglik_variant = 1;
+    // 1 = a log-lik of the current factor and field right after a sweep sums the sweep's residual r instead of rebuilding it
+    // (default); 0 = always the full pass (comparison)
+    bool loglik_from_residual = true;
     int n_slots = 0;                       // padded length of the level-ordered row list
     int solve_ctas_per_sm = 1;             // window of the sync-free solve = n_sm * this * 256 rows
     int solve_window_ctas = 0;             // if > 0: absolute number of CTAs (overrides the per-SM setting)
@@ -278,6 +281,10 @@ struct Ctx {
     size_t h_stage_n = 0;
 
     int cur = 0;                      // which linv buffer is the current factor (slot 0); the other one is the proposal
+    // d_r = linv[cur] (d_field - r_beta0): set by refresh_r and kept by the sweeps that follow it (they patch r with the same beta_0);
+    // cleared on entry to every ABI call that is not known to leave d_field, d_r, linv[cur] and cur alone (get_ctx)
+    bool r_valid = false;
+    double r_beta0 = 0.0;
     bool have_factor[2] = {false, false};
     bool committed = false;           // valT / pd correspond to linv[cur]
     bool have_field = false, have_obs = false, have_newfield = false;
@@ -304,11 +311,14 @@ struct Ctx {
 static std::mutex g_ctx_mu;
 static std::vector<Ctx *> g_ctx;
 
-static Ctx *get_ctx(const int *id) {
+// keep_r: the calling entry point leaves the residual's validity as it is (reads only, or sets it itself after a sweep); every
+// other entry point may change the field, the residual or the current factor, so it forgets that r is current
+static Ctx *get_ctx(const int *id, bool keep_r = false) {
     REQUIRE(id != nullptr, "null ctx_id");
     std::lock_guard<std::mutex> lk(g_ctx_mu);
     REQUIRE(*id >= 0 && *id < (int)g_ctx.size() && g_ctx[*id] != nullptr, "unknown context id %d", *id);
     Ctx *c = g_ctx[*id];
+    if (!keep_r) c->r_valid = false;
     return c;
 }
 
@@ -528,9 +538,18 @@ static bool launch_loglik_tma(Ctx *c, const double *linv, const double *field, d
     return true;
 }
 
-// partial sums -> d_scalars[off..off+1]
-static void op_loglik_sums(Ctx *c, const double *linv, const double *field, double shift, int scal_off) {
+// partial sums -> d_scalars[off..off+1].  allow_residual: the caller accepts the sums taken from the sweep's residual when it is
+// current for exactly this factor, field and beta_0 (an unsharded context); they differ from the full pass by the rounding the
+// sweep's incremental updates of r accumulated
+static void op_loglik_sums(Ctx *c, const double *linv, const double *field, double shift, int scal_off, bool allow_residual) {
     int blocks = std::min(kReduceBlocks, (c->n + 255) / 256);
+    if (allow_residual && c->loglik_from_residual && !c->sharded && c->r_valid && linv == c->d_linv[c->cur].p && field == c->d_field.p &&
+        std::memcmp(&shift, &c->r_beta0, sizeof(double)) == 0) {
+        loglik_residual_kernel<<<blocks, 256, 0, c->stream>>>(linv, c->d_r.p, c->n, reinterpret_cast<double2 *>(c->d_partials.p),
+                                                              reinterpret_cast<unsigned int *>(c->d_ticket.p + 1), c->d_scalars.p + scal_off);
+        LAUNCHED(c);
+        return;
+    }
     bool done = false;
     if (c->loglik_variant == 0) {   // TMA-staged ring (specialised neighbour counts only)
         if (c->M == 6) done = launch_loglik_tma<6, 4>(c, linv, field, shift, &blocks);
@@ -863,7 +882,11 @@ static void ensure_zbuf(Ctx *c, size_t count) {
     if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; }  // zbuf pointer is baked in
 }
 
-static void refresh_r(Ctx *c, double beta0) { op_spmv(c, c->d_linv[c->cur].p, c->d_field.p, beta0, c->d_r.p); }
+static void refresh_r(Ctx *c, double beta0) {
+    op_spmv(c, c->d_linv[c->cur].p, c->d_field.p, beta0, c->d_r.p);
+    c->r_valid = !c->sharded;   // a sharded field's ghost rows are not kept current by its own sweep
+    c->r_beta0 = beta0;
+}
 
 // ---- dense products with the resident design matrices (update_Gaussian.R:226-246) ----
 static const int kAtbRowsPerChunk = 4096;
@@ -1376,7 +1399,8 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
     if (!c->partial_rows.empty()) c->d_partial_rows.upload(c->partial_rows, s);
     c->d_nbad.alloc(8);   // [0] rows with a non-PD block, [1] wait timed out (1 solve, 2 halo / reduction), [3..5] which solve row waited for what
     CK(cudaMemsetAsync(c->d_nbad.p, 0, 8 * sizeof(int), s));
-    c->d_ticket.alloc(1);
+    c->d_ticket.alloc(2);   // [0] the triangular solve's chunk tickets, [1] the residual log-lik's CTA count (back to 0 after every launch)
+    CK(cudaMemsetAsync(c->d_ticket.p, 0, 2 * sizeof(int), s));
     c->d_rows_padded.upload(rows_padded, s);
     {   // level-ordered copies for the triangular solve: static neighbour table now, factor values at every factor build
         std::vector<int> lpos(n, -1), nn_lvl((size_t)c->n_slots * M, -1);
@@ -1533,6 +1557,7 @@ void nngp_ctx_set_option(const int *ctx_id, const int *key, const int *value, in
         case NNGP_OPT_USE_GRAPH: c->use_graph = (*value != 0); break;
         case NNGP_OPT_SOLVE_CTAS_PER_SM: REQUIRE(*value >= 1 && *value <= 8, "solve CTAs per SM must be 1..8"); c->solve_ctas_per_sm = *value; break;
         case NNGP_OPT_LOGLIK_VARIANT: REQUIRE(*value >= 0 && *value <= 1, "loglik variant must be 0..1"); c->loglik_variant = *value; break;
+        case NNGP_OPT_LOGLIK_FROM_RESIDUAL: c->loglik_from_residual = (*value != 0); break;
         case NNGP_OPT_MATERN_TABLE: c->matern_table = (*value != 0); break;
         case NNGP_OPT_COMMIT_VARIANT: REQUIRE(*value >= 0 && *value <= 1, "commit variant must be 0..1"); c->commit_variant = *value; break;
         case NNGP_OPT_SOLVE_WINDOW_CTAS: REQUIRE(*value >= 0 && *value <= 4096, "solve window must be 0..4096 CTAs"); c->solve_window_ctas = *value; break;
@@ -1697,7 +1722,7 @@ void nngp_field_set(const int *ctx_id, const double *field, int *status) {
 
 void nngp_field_get(const int *ctx_id, double *field, int *status) {
     ABI_BEGIN
-    Ctx *c = get_ctx(ctx_id);
+    Ctx *c = get_ctx(ctx_id, true);
     REQUIRE(field != nullptr, "null field");
     NEED(c->have_field, "nngp_field_get: no field on the device");
     use(c);
@@ -1724,12 +1749,12 @@ void nngp_obs_set(const int *ctx_id, const double *y_minus_xb, int *status) {
 
 void nngp_loglik(const int *ctx_id, const int *slot, const double *beta_0, const double *log_scale, double *ll, int *status) {
     ABI_BEGIN
-    Ctx *c = get_ctx(ctx_id);
+    Ctx *c = get_ctx(ctx_id, true);
     REQUIRE(slot && beta_0 && log_scale && ll && (*slot == 0 || *slot == 1), "nngp_loglik: bad argument");
     NEED(c->have_slot(*slot), "nngp_loglik: that slot holds no factor");
     NEED(c->have_field, "nngp_loglik: no field on the device");
     use(c);
-    op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, 0);
+    op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, 0, true);
     fetch_scalars(c, 2);
     *ll = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], *log_scale);
     ABI_END
@@ -1742,7 +1767,7 @@ void nngp_loglik_host(const int *ctx_id, const int *slot, const double *z, const
     NEED(c->have_slot(*slot), "nngp_loglik_host: that slot holds no factor");
     use(c);
     upload_site_vector(c, z, c->d_tmp1.p);
-    op_loglik_sums(c, c->linv_slot(*slot), c->d_tmp1.p, 0.0, 0);
+    op_loglik_sums(c, c->linv_slot(*slot), c->d_tmp1.p, 0.0, 0, false);
     fetch_scalars(c, 2);
     *ll = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], *log_scale);
     ABI_END
@@ -1851,12 +1876,12 @@ void nngp_sweep_loglik_host(const int *ctx_id, const int *n_sweeps, const double
         CK(cudaEventRecord(c->ev_copy, c->stream));
         CK(cudaStreamWaitEvent(c->copy_stream, c->ev_copy, 0));
         CK(cudaMemcpyAsync(field_io, c->d_io.p, sizeof(double) * c->n, cudaMemcpyDeviceToHost, c->copy_stream));
-        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, 0);
+        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, 0, true);
         CK(cudaMemcpyAsync(c->h_pinned, c->d_scalars.p, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
         CK(cudaStreamSynchronize(c->stream));
         CK(cudaStreamSynchronize(c->copy_stream));
     } else {
-        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, 0);
+        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, 0, true);
         CK(cudaMemcpyAsync(c->h_pinned, c->d_scalars.p, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
         download_site_vector(c, c->d_field.p, field_io);   // synchronises
     }
@@ -2041,7 +2066,7 @@ void nngp_shard_group_loglik(const int *ctx_ids, const int *world, const int *sl
         NEED(cs[h]->sharded && (cs[h]->p2p || W == 1), "nngp_shard_group_loglik: the contexts are not connected (nngp_shard_connect_local)");
         NEED(cs[h]->have_slot(*slot) && cs[h]->have_field, "nngp_shard_group_loglik: factor and field must be set first");
     }
-    for (Ctx *c : cs) { use(c); op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, 0); }
+    for (Ctx *c : cs) { use(c); op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, 0, false); }
     for (int h = 0; h < W; h++) {
         Ctx *c = cs[h];
         use(c);
@@ -2311,6 +2336,9 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
     REQUIRE(ns >= 1 && ns <= 5 && n_iter >= 0 && n_chromatic >= 0, "nngp_chain_run: bad sizes");
     NEED(c->can_sweep, "this context was created without a colouring (all-zero coloring): it cannot run Gibbs sweeps");
     use(c);
+    // the loop refreshes r before its sweeps and changes the field and the factor after them: however it ends, r is not left
+    // marked current
+    struct ForgetR { Ctx *c; ~ForgetR() { c->r_valid = false; } } forget_r{c};
     // regressors: beta, the interweaving matrices (:77-83) and scratch for the (p+1)- and q-vectors
     const int reg_p = reg ? c->reg_p : 0, reg_q = reg ? c->reg_q : 0, P1 = reg_p + 1;
     std::vector<double> beta, iw_cov, iw_chol, gvec, bmean, zz, innov, coefl;
@@ -2432,8 +2460,8 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         if (std::exp(new_log_scale) < var_y) {                                    // :167
             for (int k = 0; k < ns; k++) new_shape[k] = shape[k] + innovation[1 + k];
             op_factor_build(c, NNGP_SLOT_PROPOSAL, to_covparms(new_shape));      // :179
-            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_PROPOSAL), c->d_field.p, beta_0, 0);
-            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, beta_0, 2);
+            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_PROPOSAL), c->d_field.p, beta_0, 0, false);
+            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, beta_0, 2, false);
             fetch_scalars(c, 4);
             const int bad_s = n_bad();
             const double GP_ratio = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], new_log_scale) -
@@ -2855,7 +2883,7 @@ void nngp_records_summary(const int *ctx_id, const int *first_row, const int *n_
 
 void nngp_time_op(const int *ctx_id, const int *op_, const int *reps_, const int *flush_l2_, double *ms_out, int *launches_out, int *status) {
     ABI_BEGIN
-    Ctx *c = get_ctx(ctx_id);
+    Ctx *c = get_ctx(ctx_id, true);   // no timed op writes the field, r or the current factor; the sweeps keep r current
     NEED(!c->sharded || *op_ != 4 || c->world == 1 || (c->p2p && c->can_solve), "nngp_time_op: the triangular solve of a sharded context needs the peer-to-peer transport");
     REQUIRE(op_ && reps_ && flush_l2_ && ms_out && *reps_ >= 1, "nngp_time_op: bad argument");
     const int op = *op_;
@@ -2878,14 +2906,14 @@ void nngp_time_op(const int *ctx_id, const int *op_, const int *reps_, const int
         CK(cudaEventRecord(c->ev0, c->stream));
         switch (op) {
             case 0: op_factor_build(c, NNGP_SLOT_PROPOSAL, c->last_cc); break;
-            case 1: op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0); break;
+            case 1: op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, false); break;
             case 2: op_sweeps(c, 1); c->sweep_counter++; break;
             case 3: op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, c->d_tmp1.p); break;
             case 4: op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, c->d_tmp1.p);
                     op_sptrsv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_tmp1.p, c->d_tmp2.p, nullptr, 0.0, 1.0); break;
             case 5: op_commit(c); break;
             case 6: op_sweeps(c, 1); c->sweep_counter++;
-                    op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0); break;
+                    op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, true); break;
             default: REQUIRE(false, "nngp_time_op: unknown op %d", op);
         }
         CK(cudaEventRecord(c->ev1, c->stream));
@@ -2909,7 +2937,7 @@ void nngp_time_op_group(const int *ctx_ids, const int *n_ctx, const int *op_, co
     const int nc = *n_ctx;
     std::vector<Ctx *> cs(nc);
     for (int k = 0; k < nc; k++) {
-        cs[k] = get_ctx(ctx_ids + k);
+        cs[k] = get_ctx(ctx_ids + k, true);
         NEED(!cs[k]->sharded && cs[k]->can_sweep && cs[k]->have_slot(NNGP_SLOT_CURRENT) && cs[k]->have_field && cs[k]->have_obs, "nngp_time_op_group: every context needs a factor, a field and observations");
         REQUIRE(cs[k]->device == cs[0]->device, "nngp_time_op_group: the contexts must share a device");
     }
@@ -2930,7 +2958,7 @@ void nngp_time_op_group(const int *ctx_ids, const int *n_ctx, const int *op_, co
         for (Ctx *c : cs) {
             op_sweeps(c, 1);
             c->sweep_counter++;
-            if (*op_ == 6) op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0);
+            if (*op_ == 6) op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, true);
         }
     for (Ctx *c : cs) CK(cudaEventRecord(c->ev1, c->stream));
     double worst = 0.0;

@@ -225,6 +225,9 @@ void nngp_host_shard_plan_get(const int *plan_id, double *locs, int *NNarray, in
 #define NNGP_OPT_SHARD_GHOST_FIRST 12 /* ... 0 = at the end of the grid (default); 1 = at its head, resident before the peers' values land; 2 = per colour: head iff tiles and ghost CTAs are co-resident; default 0 (measured: 167 / 180 / 168 us on 2 GPUs x 1M sites) */
 #define NNGP_OPT_FACTOR_VARIANT 14    /* factor build at m = 20: 0 = one thread per row, as for m <= 10 (default); 1 = one warp per row (measured slower for the exponential family, equal for Matern) */
 #define NNGP_OPT_LOGLIK_VARIANT 10    /* log-lik pass: 1 = plain coalesced loads (default, faster); 0 = TMA-staged shared-memory ring (cp.async.bulk + mbarrier) */
+#define NNGP_OPT_LOGLIK_FROM_RESIDUAL 15 /* 1 = nngp_loglik (current factor, device field) right after nngp_gibbs_sweep with the same beta_0, and
+                                          * nngp_sweep_loglik_host, sum the residual linv (field - beta_0) the sweep keeps instead of the full pass
+                                          * (default; equal up to the rounding of the sweep's updates of it); 0 = always the full pass */
 void nngp_ctx_set_option(const int *ctx_id, const int *key, const int *value, int *status);
 /* development aid: one sweep of a connected sharded field with six time stamps per colour (first tile past its wait, last boundary
  * push, first / last ghost value seen, last ghost site patched, last tile done); out_ns[n_colors][6], ns, -1 = not set.  Every rank
