@@ -31,11 +31,13 @@ def make_problem(n, m, d=2, seed=0, n_extra_obs=0, drop_obs_frac=0.0, locs=None)
                 obs_per_loc=obs_per_loc, y=y, field=field, n=n, m=m, d=d)
 
 
-def make_regression_problem(n, m, seed=0, n_extra_obs=0, p_locs=2, p_obs=1, range_=0.1):
+def make_regression_problem(n, m, seed=0, n_extra_obs=0, p_locs=2, p_obs=1, range_=0.1, xlocs=None):
     """A Gaussian NNGP model WITH regressors as mcmc_nngp_initialize prepares it (initialize.R:116-137): X$X = centred
     cbind(X_locs[locs_match], X_obs) without intercept, X$locs = 1..p_locs, solve_1XT1X / chol_solve_1XT1X (upper factor),
     hctam_scol_1 = first observation of every site; y = beta_0 + X beta + w[locs_match] + noise with w drawn from the prior
-    by the host utilities (no oracle, no GPU)."""
+    by the host utilities (no oracle, no GPU).
+    xlocs (1-based, p_locs distinct columns of 1..p_locs + p_obs): X$locs in that order instead of the prefix; the l-th
+    location-level column goes to column xlocs[l] of X$X and the observation-level columns fill the others in order."""
     P = make_problem(n, m, seed=seed, n_extra_obs=n_extra_obs)
     rng, lm = P["rng"], P["locs_match"] - 1
     n_obs = P["n_obs"]
@@ -46,6 +48,15 @@ def make_regression_problem(n, m, seed=0, n_extra_obs=0, p_locs=2, p_obs=1, rang
     if p_obs:
         cols.append(rng.standard_normal((n_obs, p_obs)))
     X = np.column_stack(cols)
+    if xlocs is None:
+        xlocs = np.arange(1, p_locs + 1)
+    else:
+        xlocs = np.asarray(xlocs)
+        assert xlocs.size == p_locs and np.unique(xlocs).size == p_locs and xlocs.min() >= 1 and xlocs.max() <= X.shape[1]
+        order = np.empty(X.shape[1], dtype=np.int64)
+        order[xlocs - 1] = np.arange(p_locs)
+        order[np.setdiff1d(np.arange(X.shape[1]), xlocs - 1)] = np.arange(p_locs, X.shape[1])
+        X = X[:, order]
     X = X - X.mean(axis=0)                                                       # initialize.R:132
     one = np.column_stack([np.ones(n_obs), X])
     S = np.linalg.inv(one.T @ one)                                               # :135
@@ -56,9 +67,35 @@ def make_regression_problem(n, m, seed=0, n_extra_obs=0, p_locs=2, p_obs=1, rang
     # a smooth field with roughly the right range (exact prior draws are not needed for these tests)
     w = np.sin(P["locs"][:, 0] / range_) * np.cos(P["locs"][:, 1] / range_) + 0.3 * rng.standard_normal(n)
     y = 0.7 + X @ beta_true + w[lm] + np.sqrt(0.1) * rng.standard_normal(n_obs)
-    P.update(X=X, xlocs=np.arange(1, p_locs + 1, dtype=np.int32), first_obs=(first + 1).astype(np.int32), solve_1XT1X=S,
+    P.update(X=X, xlocs=xlocs.astype(np.int32), first_obs=(first + 1).astype(np.int32), solve_1XT1X=S,
              chol_solve_1XT1X=np.linalg.cholesky(S).T, beta_true=beta_true, y=y, w=w)
     return P
+
+
+def assert_regression_chain_matches(dev, ora, X, y, locs_match, label, tol_rec=1e-8, tol_field=1e-7, tol_ssr=1e-7):
+    """A device chain with regressors against the oracle chain driven by the same R stream.
+    dev = (params, records, beta records, field records, accepts, final field, SSR of the context's y - X beta - field);
+    ora = O.update_gaussian_chain(..., regressors=...) = (params, field, records, field records, accepts, beta records).
+    Same accept/reject sequence with at least one accept (each accept rebuilds the interweaving matrices), records, beta records
+    and the final beta within tol_rec, fields within tol_field, the SSR within tol_ssr relative.  Prints the largest
+    differences (pytest -rP shows them)."""
+    pg, recg, brecg, frecg, accg, fg, ssr_g = dev
+    po, fo, reco, freco, acco, breco = ora
+    lm = np.asarray(locs_match) - 1
+    ssr_o = float(np.sum((y - X @ po["beta"] - fo[lm]) ** 2))
+    gaps = dict(records=np.max(np.abs(recg - reco)), beta_records=np.max(np.abs(brecg - breco)),
+                beta=np.max(np.abs(pg["beta"] - po["beta"])), field=np.max(np.abs(fg - fo)),
+                field_records=np.max(np.abs(frecg - freco)), ssr_rel=abs(ssr_g - ssr_o) / ssr_o)
+    print(f"{label}: accepts {int(accg.sum())} of {accg.size}; " + ", ".join(f"{k} {v:.2e}" for k, v in gaps.items()))
+    flips = np.argwhere(accg != acco)
+    assert flips.size == 0, f"{label}: accept/reject differs at (iteration - 1, step) {flips[:5].tolist()}"
+    assert accg.sum() > 0, label
+    for k in ("records", "beta_records", "beta"):
+        assert gaps[k] < tol_rec, (label, k, gaps[k], tol_rec)
+    for k in ("field", "field_records"):
+        assert gaps[k] < tol_field, (label, k, gaps[k], tol_field)
+    assert gaps["ssr_rel"] < tol_ssr, (label, gaps["ssr_rel"], tol_ssr)
+    assert abs(pg["logvar_sufficient"] - po["logvar_sufficient"]) < 1e-12, label
 
 
 # ---------------------------------------------------------------------------------------------------------------------------

@@ -321,43 +321,61 @@ def test_chain_run_matches_oracle_chain_with_r_stream(covfun, shape):
     assert abs(pg["logvar_ancillary"] - po["logvar_ancillary"]) < 1e-12
 
 
-@pytest.mark.parametrize("p_locs,p_obs,extra,covfun,shape", [(2, 1, 300, "exponential_isotropic", [np.log(0.1)]),
-                                                             (0, 3, 0, "exponential_isotropic", [np.log(0.1)]),
-                                                             (3, 0, 100, "matern_isotropic", [np.log(0.1), 0.3]),
-                                                             (20, 4, 50, "exponential_isotropic", [np.log(0.1)])])
-def test_chain_run_regressors_matches_oracle_chain_with_r_stream(p_locs, p_obs, extra, covfun, shape):
+REGRESSOR_CHAIN_CASES = [   # n sites, p_locs, p_obs, extra observations, covfun, shape, X$locs (None: 1..p_locs)
+    (1500, 2, 1, 300, "exponential_isotropic", [np.log(0.1)], None),
+    (1500, 0, 3, 0, "exponential_isotropic", [np.log(0.1)], None),
+    (1500, 3, 0, 100, "matern_isotropic", [np.log(0.1), 0.3], None),
+    (1500, 20, 4, 50, "exponential_isotropic", [np.log(0.1)], None),
+    # around op_atb's row chunks (kAtbRowsPerChunk = 4096 rows, nngp_b200.cu): one full chunk of observations with p + 1 = 17 (one
+    # column past a 16-wide tile); 4097 observations and 4097 sites with q = 17, so both products get a second chunk of one row;
+    # 13 000 observations over 10 000 sites with 80 columns (4 and 3 chunks, 6 x 2 tiles of the interweaving product)
+    (4000, 4, 12, 96, "exponential_isotropic", [np.log(0.1)], None),
+    (4097, 16, 2, 0, "matern_isotropic", [np.log(0.1), 0.3], None),
+    (10000, 20, 60, 3000, "exponential_isotropic", [np.log(0.1)], None),
+    (10000, 20, 60, 3000, "matern_isotropic", [np.log(0.05), -0.5], None),
+    # X$locs not a prefix of X's columns: the interweaving step reads and writes beta through the X$locs map
+    (1500, 2, 2, 100, "exponential_isotropic", [np.log(0.1)], [3, 1]),
+]
+
+
+def _regressor_case_id(i, case):
+    """pytest's id of (p_locs, p_obs, extra, covfun, shape), with n and X$locs appended where they are not 1500 and a prefix"""
+    n, p_locs, p_obs, extra, covfun, _, xlocs = case
+    s = f"{p_locs}-{p_obs}-{extra}-{covfun}-shape{i}"
+    return s + (f"-n{n}" if n != 1500 else "") + (f"-xlocs{'_'.join(map(str, xlocs))}" if xlocs else "")
+
+
+@pytest.mark.parametrize("n,p_locs,p_obs,extra,covfun,shape,xlocs", REGRESSOR_CHAIN_CASES,
+                         ids=[_regressor_case_id(i, c) for i, c in enumerate(REGRESSOR_CHAIN_CASES)])
+def test_chain_run_regressors_matches_oracle_chain_with_r_stream(n, p_locs, p_obs, extra, covfun, shape, xlocs):
     """nngp_chain_run_regressors (update_Gaussian.R:101-314 with the regression block :226-250 on the device: X resident in
     HBM, crossprod()s as streaming A^T B kernels, interweaving matrices refreshed on every accept) against the oracle chain
     (itself checked against the dense transcription of the R loop, tests/test_oracle_golden.py), both driven by R's stream."""
-    from problems import make_regression_problem
-    n, m, n_iter = 1500, 5, 50
-    P = make_regression_problem(n, m, seed=23, n_extra_obs=extra, p_locs=p_locs, p_obs=p_obs)
-    p0 = dict(shape=shape, beta_0=0.5, log_scale=-0.2, log_noise_variance=np.log(0.15), logvar_sufficient=-2.0, logvar_ancillary=-2.0)
+    from problems import assert_regression_chain_matches
+    m, n_iter = 5, 50
+    P = make_regression_problem(n, m, seed=23, n_extra_obs=extra, p_locs=p_locs, p_obs=p_obs, xlocs=xlocs)
+    K, chunks = 4096, lambda rows: -(-rows // 4096)    # kAtbRowsPerChunk (nngp_b200.cu): op_atb sums partials over chunks of K rows
+    if n == 4000:      # exactly one full chunk of observations, p + 1 = 17
+        assert P["n_obs"] == K and P["X"].shape[1] + 1 == 17
+    elif n == 4097:    # a second chunk of one row for the observations and for the sites, q = 17
+        assert P["n_obs"] == K + 1 and n == K + 1 and p_locs + 1 == 17
+    elif n == 10000:   # 4 chunks of observations, 3 of sites
+        assert chunks(P["n_obs"]) == 4 and chunks(n) == 3
+    p0 =dict(shape=shape, beta_0=0.5, log_scale=-0.2, log_noise_variance=np.log(0.15), logvar_sufficient=-2.0, logvar_ancillary=-2.0)
     beta0 = 0.1 * np.ones(P["X"].shape[1])
     field0 = 0.5 + P["w"]
     reg = dict(X=P["X"], xlocs=P["xlocs"], first_obs=P["first_obs"], solve_1XT1X=P["solve_1XT1X"],
                chol_solve_1XT1X=P["chol_solve_1XT1X"], beta=beta0)
-    po, fo, reco, freco, acco, breco = O.update_gaussian_chain(P["locs"], P["NNarray"], P["coloring"], P["locs_match"], P["obs_per_loc"],
-                                                               P["y"], covfun, p0, field0, n_iter, 0.5, 2, 0, 3, 1, regressors=reg)
+    ora = O.update_gaussian_chain(P["locs"], P["NNarray"], P["coloring"], P["locs_match"], P["obs_per_loc"],
+                                  P["y"], covfun, p0, field0, n_iter, 0.5, 2, 0, 3, 1, regressors=reg)
     var_y = float(np.var(P["y"], ddof=1))
     with nb.NNGPContext(P["locs"], P["NNarray"], P["coloring"], P["locs_match"], covfun) as ctx:
         ctx.regressors_set(P["X"], P["y"], xlocs=P["xlocs"], first_obs=P["first_obs"])
         ctx.field_set(field0)
-        pg, recg, brecg, frecg, accg = ctx.chain_run_regressors(p0, beta0, P["solve_1XT1X"], P["chol_solve_1XT1X"], n_iter, var_y, thin=0.5,
-                                                                n_chromatic=2, iter_start=0, chain_index=3, rng_mode=nb.RNG_SUPPLIED)
-        fg = ctx.field_get()
-        ssr_g = ctx.ssr()                                      # the context's y - X beta corresponds to the final beta
-    assert np.array_equal(accg, acco)
-    assert accg.sum() > 0
-    assert np.max(np.abs(recg - reco)) < 1e-8
-    assert np.max(np.abs(brecg - breco)) < 1e-8
-    assert np.max(np.abs(fg - fo)) < 1e-7
-    assert np.max(np.abs(frecg - freco)) < 1e-7
-    assert np.max(np.abs(pg["beta"] - po["beta"])) < 1e-8
-    assert abs(pg["logvar_sufficient"] - po["logvar_sufficient"]) < 1e-12
-    lm = P["locs_match"] - 1
-    ssr_o = float(np.sum((P["y"] - P["X"] @ po["beta"] - fo[lm]) ** 2))
-    assert abs(ssr_g - ssr_o) < 1e-7 * ssr_o
+        dev = ctx.chain_run_regressors(p0, beta0, P["solve_1XT1X"], P["chol_solve_1XT1X"], n_iter, var_y, thin=0.5,
+                                       n_chromatic=2, iter_start=0, chain_index=3, rng_mode=nb.RNG_SUPPLIED)
+        dev = dev + (ctx.field_get(), ctx.ssr())               # the context's y - X beta corresponds to the final beta
+    assert_regression_chain_matches(dev, ora, P["X"], P["y"], P["locs_match"], f"n={n} p_locs={p_locs} p_obs={p_obs} {covfun}")
 
 
 def test_regressor_error_paths():
