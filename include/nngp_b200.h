@@ -51,6 +51,15 @@ extern "C" {
 /* rng_mode for the field draws of the chromatic sweep */
 #define NNGP_RNG_SUPPLIED 0 /* caller passes the normals (R's rnorm stream): bit-comparable with the reference order */
 #define NNGP_RNG_PHILOX 1   /* counter-based Philox4x32-10 keyed by (seed, sweep counter, global site id) */
+/* The Philox stream.  The normal of site g (0-based reference index; global on a sharded field) in the sweep at counter k under
+ * seed s is Philox4x32-10 with counter (g, k & 0xffffffff, k >> 32, 0x4e4e4750) and key (s & 0xffffffff, (s >> 32) ^ 0x5eed5eed),
+ * s = (uint64_t)(int64_t)seed; from its output words a = (x << 32) | y, b = (z << 32) | w, u1 = ((a >> 11) + 0.5) 2^-53, u2 likewise
+ * from b, and the normal is sqrt(-2 log u1) cospi(2 u2).  Each context keeps a sweep counter that starts at 0 when the context is
+ * created and advances by one for every sweep run on it, whatever the rng_mode: nngp_gibbs_sweep and nngp_sweep_loglik_host by
+ * n_sweeps, nngp_chain_run* by n_iter * n_chromatic, nngp_time_op ops 2 and 6 by one per repetition, nngp_time_op_group by
+ * reps + 1 on each context, the shard colour-stepping entry points by one per sweep.  nngp_chain_run* take
+ * seed = (iter_start << 20) ^ chain_index, so nngp_gibbs_sweep with seed s draws under the same key as nngp_chain_run with
+ * iter_start = 0 and chain_index = s.  tests/philox_reference.py restates all of this. */
 
 /* internal site layout (performance knob; results are layout-independent up to FP64 summation order) */
 #define NNGP_LAYOUT_COLOR 1        /* vectors stored colour-major, reference order inside a colour */
@@ -295,8 +304,8 @@ void nngp_sptrsv(const int *ctx_id, const int *slot, const double *b, double *x,
 /* n_sweeps chromatic Gibbs sweeps of the latent field (Scripts/mcmc_nngp_update_Gaussian.R:257-275) with the current
  * factor.  rng_mode NNGP_RNG_SUPPLIED: z holds n_sweeps * n normals, sweep-major, each sweep in the order in which the
  * reference's rnorm(length(selected_locs)) calls hand them out (colour 1..K, sites ascending inside a colour).
- * NNGP_RNG_PHILOX: z is ignored (may be NULL); seed/stream pick the Philox key, and the library advances a per-context
- * sweep counter. */
+ * NNGP_RNG_PHILOX: z is ignored (may be NULL); seed picks the Philox key, and sweep j of the call (j = 0 .. n_sweeps - 1) draws at
+ * the context's sweep counter + j (see NNGP_RNG_PHILOX).  Either mode advances the counter by n_sweeps. */
 void nngp_gibbs_sweep(const int *ctx_id, const int *n_sweeps, const double *beta_0, const double *log_scale,
                       const double *log_noise_variance, const int *rng_mode, const double *z, const double *seed,
                       int *status);
@@ -326,8 +335,10 @@ void nngp_field_init(const int *ctx_id, const int *slot, const double *beta_0, c
  * records_out: n_iter x (3 + k) column-major [beta_0, log_scale, log_noise_variance, shape...]
  * field_records_out: round(n_iter * thin) x n column-major, or NULL
  * rng_mode NNGP_RNG_SUPPLIED reproduces R's stream (set.seed(iter_start + chain_index), Mersenne-Twister + inversion)
- * for every draw including the field normals; NNGP_RNG_PHILOX uses R's stream for the scalar draws and Philox for the
- * field. */
+ * for every draw including the field normals; NNGP_RNG_PHILOX uses R's stream for the scalar draws (skipping the field's rnorm()
+ * calls, update_Gaussian.R:75 included) and Philox for the field: seed (iter_start << 20) ^ chain_index, iteration i's sweeps at
+ * counters c0 + (i - 1) n_chromatic .. c0 + i n_chromatic - 1, c0 = the context's sweep counter when the call starts (see
+ * NNGP_RNG_PHILOX). */
 void nngp_chain_run(const int *ctx_id, const int *n_shape, double *params_io, const int *n_iter, const double *thin,
                     const int *n_chromatic, const int *iter_start, const int *chain_index, const int *rng_mode,
                     const double *var_y, double *records_out, double *field_records_out, int *accept_out, int *status);

@@ -595,6 +595,68 @@ int oracle_update_gaussian_chain_x(const double *locs, int n, int d, const int *
                                    int chain_index, int sweep_form, double *records, double *field_records,
                                    int *accept_records, const oracle_regressors *reg)
 {
+    return oracle_update_gaussian_chain_rng(locs, n, d, NNarray, m, coloring, n_colors, locs_match, n_obs, obs_per_loc,
+                                            observed_field, covfun, p, field, n_iterations_update, field_thinning, n_chromatic,
+                                            iter_start, chain_index, sweep_form, records, field_records, accept_records, reg,
+                                            ORACLE_RNG_R, 0, 0);
+}
+
+/* ------------------------------------------------------------------------------------------------------------- */
+/* the product's Philox normals                                                                                    */
+/* ------------------------------------------------------------------------------------------------------------- */
+
+void oracle_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4])
+{
+    uint32_t x = ctr[0], y = ctr[1], z = ctr[2], w = ctr[3], k0 = key[0], k1 = key[1];
+    for (int r = 0; r < 10; r++) {
+        uint64_t p0 = (uint64_t)0xD2511F53u * x, p1 = (uint64_t)0xCD9E8D57u * z;
+        uint32_t nx = (uint32_t)(p1 >> 32) ^ y ^ k0, ny = (uint32_t)p1, nz = (uint32_t)(p0 >> 32) ^ w ^ k1, nw = (uint32_t)p0;
+        x = nx; y = ny; z = nz; w = nw;
+        k0 += 0x9E3779B9u;
+        k1 += 0xBB67AE85u;
+    }
+    out[0] = x; out[1] = y; out[2] = z; out[3] = w;
+}
+
+void oracle_philox_key(int64_t seed, uint32_t key[2])
+{
+    uint64_t s = (uint64_t)seed;
+    key[0] = (uint32_t)(s & 0xffffffffu);
+    key[1] = (uint32_t)(s >> 32) ^ 0x5eed5eedu;
+}
+
+double oracle_philox_normal(uint32_t site, uint64_t counter, uint32_t k0, uint32_t k1)
+{
+    uint32_t c[4] = {site, (uint32_t)counter, (uint32_t)(counter >> 32), 0x4e4e4750u}, k[2] = {k0, k1}, r[4];
+    oracle_philox4x32_10(c, k, r);
+    uint64_t a = ((uint64_t)r[0] << 32) | r[1], b = ((uint64_t)r[2] << 32) | r[3];
+    double u1 = ((double)(a >> 11) + 0.5) * 1.1102230246251565e-16;   /* 2^-53 */
+    double u2 = ((double)(b >> 11) + 0.5) * 1.1102230246251565e-16;
+    return sqrt(-2.0 * log(u1)) * cos(2.0 * M_PI * u2);
+}
+
+/* sites listed in hand-out order (color_buckets) */
+static void philox_fill(const int *order, int n, uint64_t counter, uint32_t k0, uint32_t k1, double *z)
+{
+    for (int q = 0; q < n; q++) z[q] = oracle_philox_normal((uint32_t)order[q], counter, k0, k1);
+}
+
+void oracle_philox_handout(const int *coloring, int n, int n_colors, uint64_t counter, uint32_t k0, uint32_t k1, double *z)
+{
+    int *order; int64_t *ptr;
+    color_buckets(coloring, n, n_colors, &order, &ptr);
+    philox_fill(order, n, counter, k0, k1, z);
+    free(order); free(ptr);
+}
+
+int oracle_update_gaussian_chain_rng(const double *locs, int n, int d, const int *NNarray, int m, const int *coloring,
+                                     int n_colors, const int *locs_match, int n_obs, const double *obs_per_loc,
+                                     const double *observed_field, int covfun, oracle_chain_params *p, double *field,
+                                     int n_iterations_update, double field_thinning, int n_chromatic, int iter_start,
+                                     int chain_index, int sweep_form, double *records, double *field_records,
+                                     int *accept_records, const oracle_regressors *reg, int rng_mode, int64_t philox_seed,
+                                     uint64_t sweep_counter)
+{
     const int M = m + 1, n_iter = n_iterations_update, ns = p->n_shape;
     size_t lsz = (size_t)n * M;
     double *Linv = (double *)malloc(sizeof(double) * lsz), *new_Linv = (double *)malloc(sizeof(double) * lsz);
@@ -616,7 +678,11 @@ int oracle_update_gaussian_chain_x(const double *locs, int n, int d, const int *
     shape_to_covparms(covfun, p->shape, ns, cp, &ncp);                                           /* :67-71 */
     oracle_vecchia_linv(cp, ncp, covfun, locs, n, d, NNarray, m, Linv);                          /* :72 */
     oracle_precision_diag(Linv, NNarray, n, m, precision_diag);                                  /* :74 */
-    for (int i = 0; i < n; i++) (void)r_norm_rand();                                             /* :75 current_p (dead, but consumes the stream) */
+    const int philox = rng_mode == ORACLE_RNG_PHILOX;
+    uint32_t key[2];
+    oracle_philox_key(philox_seed, key);
+    if (!philox)
+        for (int i = 0; i < n; i++) (void)r_norm_rand();                                         /* :75 current_p (dead, but consumes the stream) */
     /* regression state: X$X (n_obs x P), site-level design Xl = cbind(1, X$X[hctam_scol_1, X$locs]) (n x q) */
     const int P = reg ? reg->p : 0, P1 = P + 1, q = (reg && reg->n_xlocs > 0) ? reg->n_xlocs + 1 : 0;
     const int wlen = P1 > q ? P1 : q;
@@ -778,7 +844,8 @@ int oracle_update_gaussian_chain_x(const double *locs, int n, int d, const int *
         /* ---- chromatic sweeps :257-275 ---- */
         for (int ic = 0; ic < n_chromatic; ic++) {
             oracle_residuals_sum(locs_match, n_obs, n, observed_field, mu, residuals_sum);       /* :260 */
-            for (int q = 0; q < n; q++) z[q] = r_norm_rand(); /* rnorm(length(sel)) colour by colour = one stream */
+            if (philox) philox_fill(order, n, sweep_counter++, key[0], key[1], z);
+            else for (int q = 0; q < n; q++) z[q] = r_norm_rand(); /* rnorm(length(sel)) colour by colour = one stream */
             if (sweep_form == 0) {
                 sweep_reference(Linv, NNarray, n, m, &csc, coloring, n_colors, precision_diag, obs_per_loc,
                                 residuals_sum, p->beta_0, p->log_scale, p->log_noise_variance, z, field, tmp, tmp2);

@@ -153,6 +153,31 @@ int oracle_update_gaussian_chain_x(const double *locs, int n, int d, const int *
                                    int chain_index, int sweep_form, double *records, double *field_records,
                                    int *accept_records, const oracle_regressors *reg);
 
+/* ---- the product's on-device Philox normals (device_math.cuh philox_normal, nngp_b200.cu set_sweep_params) ---- */
+/* Philox4x32-10 (Salmon et al. 2011) */
+void oracle_philox4x32_10(const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]);
+/* key of a seed: s = (uint64)(int64)seed, key = (s & 0xffffffff, (s >> 32) ^ 0x5eed5eed) */
+void oracle_philox_key(int64_t seed, uint32_t key[2]);
+/* normal of 0-based site `site` at sweep counter `counter`: counter words (site, counter lo, counter hi, 0x4e4e4750); Box-Muller
+ * with cos(2 pi u2) (the device takes cospi(2 u2), which glibc lacks) */
+double oracle_philox_normal(uint32_t site, uint64_t counter, uint32_t k0, uint32_t k1);
+/* the n normals of one sweep in hand-out order: colour 1..n_colors, ascending site index inside a colour */
+void oracle_philox_handout(const int *coloring, int n, int n_colors, uint64_t counter, uint32_t k0, uint32_t k1, double *z);
+
+#define ORACLE_RNG_R 0
+#define ORACLE_RNG_PHILOX 1
+/* oracle_update_gaussian_chain_x with a choice of the field normals.  ORACLE_RNG_R: R's stream, as above (philox_seed and
+ * sweep_counter unused).  ORACLE_RNG_PHILOX: as nngp_chain_run* in NNGP_RNG_PHILOX mode -- the scalar draws stay on R's stream
+ * (set.seed(iter_start + chain_index)), the dead rnorm(n) of update_Gaussian.R:75 and the rnorm of every sweep are skipped, and
+ * sweep j of the call (j = 0, 1, ...) draws the Philox normals of counter sweep_counter + j under philox_seed. */
+int oracle_update_gaussian_chain_rng(const double *locs, int n, int d, const int *NNarray, int m, const int *coloring,
+                                     int n_colors, const int *locs_match, int n_obs, const double *obs_per_loc,
+                                     const double *observed_field, int covfun, oracle_chain_params *p, double *field,
+                                     int n_iterations_update, double field_thinning, int n_chromatic, int iter_start,
+                                     int chain_index, int sweep_form, double *records, double *field_records,
+                                     int *accept_records, const oracle_regressors *reg, int rng_mode, int64_t philox_seed,
+                                     uint64_t sweep_counter);
+
 #ifdef __cplusplus
 }
 #endif

@@ -59,6 +59,8 @@ def lib():
         _LIB.oracle_obs_loglik.restype = C.c_double
         _LIB.oracle_ssr.restype = C.c_double
         _LIB.oracle_moral_graph.restype = C.c_int64
+        _LIB.oracle_philox_normal.restype = C.c_double
+        _LIB.oracle_philox_normal.argtypes = [C.c_uint32, C.c_uint64, C.c_uint32, C.c_uint32]
     return _LIB
 
 
@@ -214,6 +216,38 @@ def sparse_chol_tmult(Linv, NNarray, u) -> np.ndarray:
     return out
 
 
+# ---------------------------------------------------------------- the product's Philox normals
+def philox4x32_10(counter, key) -> np.ndarray:
+    """Philox4x32-10 of four 32-bit counter words under two key words"""
+    c = (C.c_uint32 * 4)(*[int(v) & 0xFFFFFFFF for v in counter])
+    k = (C.c_uint32 * 2)(*[int(v) & 0xFFFFFFFF for v in key])
+    out = (C.c_uint32 * 4)()
+    lib().oracle_philox4x32_10(c, k, out)
+    return np.array(out[:], dtype=np.uint64)
+
+
+def philox_key(seed):
+    """(key0, key1) of a seed: s = (uint64)(int64)seed"""
+    k = (C.c_uint32 * 2)()
+    lib().oracle_philox_key(C.c_int64(int(seed)), k)
+    return k[0], k[1]
+
+
+def philox_normal(site: int, counter: int, seed) -> float:
+    k0, k1 = philox_key(seed)
+    return lib().oracle_philox_normal(site, counter, k0, k1)
+
+
+def philox_handout(coloring, counter: int, seed) -> np.ndarray:
+    """the normals of one sweep at `counter` in hand-out order (colour 1..K, ascending site inside a colour)"""
+    col = _i32(coloring)
+    k0, k1 = philox_key(seed)
+    out = np.empty(col.size)
+    lib().oracle_philox_handout(_i(col), C.c_int(col.size), C.c_int(int(col.max())), C.c_uint64(counter), C.c_uint32(k0),
+                                C.c_uint32(k1), _d(out))
+    return out
+
+
 # ---------------------------------------------------------------- sampler pieces
 def chromatic_sweep(Linv, NNarray, coloring, precision_diag_, obs_per_loc, residuals_sum, beta_0, log_scale,
                     log_noise_variance, z, field, form: str = "reference") -> np.ndarray:
@@ -279,11 +313,15 @@ class Regressors(C.Structure):
 
 def update_gaussian_chain(locs, NNarray, coloring, locs_match, obs_per_loc, observed_field, covfun_name, params: dict,
                           field, n_iterations_update, field_thinning=1.0, n_chromatic=10, iter_start=0, chain_index=1,
-                          sweep_form=0, regressors: dict | None = None):
+                          sweep_form=0, regressors: dict | None = None, rng="R", sweep_counter=0):
     """One chain of mcmc_nngp_update_Gaussian. Returns (params, field, records, field_records, accept).
     regressors = dict(X, xlocs (1-based), first_obs (1-based), solve_1XT1X, chol_solve_1XT1X, beta): the model with
     regression coefficients (update_Gaussian.R:226-250); params then also carries "beta" and the tuple gets a sixth
-    element, the beta records."""
+    element, the beta records.
+    rng = "R": every draw from R's stream, as the reference.  rng = "philox": the field normals as nngp_chain_run* draw them in
+    NNGP_RNG_PHILOX mode -- Philox under seed (iter_start << 20) ^ chain_index, sweep j of the call at counter sweep_counter + j
+    (the context's counter when the call starts), no rnorm for the field; the scalar draws stay on R's stream."""
+    assert rng in ("R", "philox")
     locs = np.asarray(locs, dtype=np.float64)
     n, d = locs.shape
     M = NNarray.shape[1]
@@ -321,14 +359,15 @@ def update_gaussian_chain(locs, NNarray, coloring, locs_match, obs_per_loc, obse
                        pd_(S), pd_(Ch), pd_(beta), pd_(brec))
         keep = [X, xl, fo, S, Ch, beta, brec]
         reg_ref = C.byref(r)
-    fn = lib().oracle_update_gaussian_chain_x
+    fn = lib().oracle_update_gaussian_chain_rng
     fn.restype = C.c_int
+    philox_seed = ((iter_start & 0xFFFFFFFF) << 20) ^ (chain_index & 0xFFFFFFFF)          # nngp_chain_run's key
     rc = fn(
         _d(_f64(locs)), C.c_int(n), C.c_int(d), _i(_i32(NNarray)), C.c_int(M - 1), _i(coloring),
         C.c_int(int(coloring.max())), _i(lm), C.c_int(lm.size), _d(_f64(obs_per_loc)), _d(_f64(observed_field)),
         C.c_int(COVFUN_IDS[covfun_name]), C.byref(p), _d(f), C.c_int(n_iter), C.c_double(field_thinning),
         C.c_int(n_chromatic), C.c_int(iter_start), C.c_int(chain_index), C.c_int(sweep_form), _d(rec), _d(frec), _i(acc),
-        reg_ref)
+        reg_ref, C.c_int(1 if rng == "philox" else 0), C.c_int64(philox_seed), C.c_uint64(sweep_counter))
     assert rc == 0
     out = dict(shape=np.array([p.shape[k] for k in range(shape.size)]), beta_0=p.beta_0, log_scale=p.log_scale,
                log_noise_variance=p.log_noise_variance, logvar_sufficient=p.logvar_sufficient,

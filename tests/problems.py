@@ -31,6 +31,23 @@ def make_problem(n, m, d=2, seed=0, n_extra_obs=0, drop_obs_frac=0.0, locs=None)
                 obs_per_loc=obs_per_loc, y=y, field=field, n=n, m=m, d=d)
 
 
+def star_problem(n, m, hubs, seed):
+    """An NNarray in which `hubs` early sites are parents of (almost) every later row: their columns hold far more than the 1024
+    entries of a sweep tile, so each becomes a single-site tile handled by the whole-CTA path (e1 - e0 > ECAP)."""
+    rng = np.random.default_rng(seed)
+    locs = rng.random((n, 2))
+    nn = nb.find_ordered_nn(locs, m)
+    for i in range(m + 1 + hubs, n):
+        h = 1 + (i % hubs)                                # 1-based hub id
+        row = nn[i, 1:]
+        if h not in row:
+            row[-1] = h                                    # replace the farthest neighbour by the hub
+    P = make_problem(n, m, seed=seed, locs=locs)
+    P["NNarray"] = nn
+    P["coloring"] = nb.greedy_coloring(nn)
+    return P
+
+
 def make_regression_problem(n, m, seed=0, n_extra_obs=0, p_locs=2, p_obs=1, range_=0.1, xlocs=None):
     """A Gaussian NNGP model WITH regressors as mcmc_nngp_initialize prepares it (initialize.R:116-137): X$X = centred
     cbind(X_locs[locs_match], X_obs) without intercept, X$locs = 1..p_locs, solve_1XT1X / chol_solve_1XT1X (upper factor),

@@ -6,7 +6,7 @@ import pytest
 
 import nngp_b200 as nb
 from oracle import oracle as O
-from problems import make_problem
+from problems import make_problem, star_problem
 
 pytestmark = pytest.mark.gpu
 TOL = 1e-10
@@ -103,23 +103,6 @@ def test_parity_matrix_on_a_maxmin_ordering(covfun, m, cp, layout):
         assert rel_vec(ctx.sptrsv(v), O.sparse_chol_solve(Lo, P["NNarray"], v)) < 1e-9
         ctx.gibbs_sweep(beta_0, ls, lnv, n_sweeps=1, z=z)
         assert rel_vec(ctx.field_get(), f_o) < TOL
-
-
-def star_problem(n, m, hubs, seed):
-    """An NNarray in which `hubs` early sites are parents of (almost) every later row: their columns hold far more than the 1024
-    entries of a sweep tile, so each becomes a single-site tile handled by the whole-CTA path (e1 - e0 > ECAP)."""
-    rng = np.random.default_rng(seed)
-    locs = rng.random((n, 2))
-    nn = nb.find_ordered_nn(locs, m)
-    for i in range(m + 1 + hubs, n):
-        h = 1 + (i % hubs)                                # 1-based hub id
-        row = nn[i, 1:]
-        if h not in row:
-            row[-1] = h                                    # replace the farthest neighbour by the hub
-    P = make_problem(n, m, seed=seed, locs=locs)
-    P["NNarray"] = nn
-    P["coloring"] = nb.greedy_coloring(nn)
-    return P
 
 
 @pytest.mark.parametrize("variant", [0, 2, 3])
