@@ -15,6 +15,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <mutex>
 #include <numeric>
 #include <string>
@@ -159,10 +160,16 @@ template <class T>
 struct DevBuf {
     T *p = nullptr;
     size_t n = 0;
-    void alloc(size_t count) {
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { release(); }
+    void alloc(size_t count) {   // after a failed allocation the buffer is empty (p == nullptr, n == 0)
         release();
+        T *q = nullptr;
+        if (count) CK(cudaMalloc(&q, count * sizeof(T)));
+        p = q;
         n = count;
-        if (count) CK(cudaMalloc(&p, count * sizeof(T)));
     }
     void upload(const std::vector<T> &h, cudaStream_t s) {
         alloc(h.size());
@@ -265,7 +272,8 @@ struct Ctx {
     DevBuf<int4> d_ginfo;
     DevBuf<unsigned long long> d_shard_tl;   // development aid: per-colour time stamps of one sharded sweep (nngp_shard_timeline)
     bool shard_tl_on = false;
-    DevBuf<double> d_sendbuf, d_recvbuf;
+    DevBuf<double> d_sendbuf;
+    double *d_recvbuf = nullptr;           // receive values of the NCCL / host-moved halo: inside p2p_area, not owned
     DevBuf<unsigned char> d_owned;         // per storage id: 1 = owned row (reductions skip ghost rows)
     DevBuf<int4> d_tiles;
     DevBuf<unsigned char> d_cloc;          // per tile (padded to 1024): local site id of every CSC entry, 255 = padding
@@ -306,7 +314,31 @@ struct Ctx {
 
     double *linv_slot(int slot) { return d_linv[slot == NNGP_SLOT_CURRENT ? cur : 1 - cur].p; }
     bool &have_slot(int slot) { return have_factor[slot == NNGP_SLOT_CURRENT ? cur : 1 - cur]; }
+    ~Ctx();
 };
+
+// the captured sweep bakes in buffer pointers and options: dropped whenever one of them changes
+static void drop_sweep_graph(Ctx *c) {
+    if (c->sweep_graph) cudaGraphExecDestroy(c->sweep_graph);
+    c->sweep_graph = nullptr;
+}
+
+// the teardown whose order matters; the DevBuf members free themselves after it
+Ctx::~Ctx() {
+    cudaSetDevice(device);
+    if (stream) cudaStreamSynchronize(stream);
+    drop_sweep_graph(this);
+    if (comm && g_nccl.ok) g_nccl.CommDestroy(comm);
+    for (int h = 0; h < 8; h++) if (peer_mapped[h]) cudaIpcCloseMemHandle(peer_mapped[h]);
+    if (p2p_area) cudaFree(p2p_area);
+    if (h_pinned) cudaFreeHost(h_pinned);
+    if (h_stage) cudaFreeHost(h_stage);
+    if (ev0) cudaEventDestroy(ev0);
+    if (ev1) cudaEventDestroy(ev1);
+    if (copy_stream) cudaStreamDestroy(copy_stream);
+    if (ev_copy) cudaEventDestroy(ev_copy);
+    if (stream) cudaStreamDestroy(stream);
+}
 
 static std::mutex g_ctx_mu;
 static std::vector<Ctx *> g_ctx;
@@ -744,7 +776,7 @@ static int launch_sweep_colors(Ctx *c) {
 
 // n_sweeps sweeps over all colours; scalar parameters are read from d_sp.  Nothing in the sequence depends on host-side values
 // (the NCCL transport excepted), so one sweep is captured once and replayed as a CUDA graph: K + 1 plain launches per sweep were
-// CPU-submission bound.
+// CPU-submission bound.  The host's sweep counter advances with every sweep enqueued, as d_sp's does when it runs.
 static void op_sweeps(Ctx *c, int n_sweeps) {
     if (n_sweeps <= 0) return;
     const bool graphable = c->use_graph && !(c->sharded && c->world > 1 && !c->p2p);
@@ -767,6 +799,7 @@ static void op_sweeps(Ctx *c, int n_sweeps) {
         }
         g_launches.fetch_add(nl, std::memory_order_relaxed);
         c->launches_in_op += nl;
+        c->sweep_counter++;
     }
 }
 
@@ -865,11 +898,11 @@ static int op_halo_exchange(Ctx *c, int col) {
         const int a = c->send_ptr[(size_t)col * W + h], b = c->send_ptr[(size_t)col * W + h + 1];
         const int ra = c->recv_ptr[(size_t)col * W + h], rb = c->recv_ptr[(size_t)col * W + h + 1];
         if (b > a) NCK(g_nccl.Send(c->d_sendbuf.p + a, (size_t)(b - a), kNcclFloat64, h, c->comm, c->stream));
-        if (rb > ra) NCK(g_nccl.Recv(c->d_recvbuf.p + ra, (size_t)(rb - ra), kNcclFloat64, h, c->comm, c->stream));
+        if (rb > ra) NCK(g_nccl.Recv(c->d_recvbuf + ra, (size_t)(rb - ra), kNcclFloat64, h, c->comm, c->stream));
     }
     NCK(g_nccl.GroupEnd());
     if (r1 > r0) {
-        halo_apply_kernel<<<(r1 - r0 + 255) / 256, 256, 0, c->stream>>>(c->d_recv_proc.p, c->d_recvbuf.p, r0, r1, c->d_colptr.p, c->d_crow.p, c->d_valT.p, c->d_psite.p, c->d_field.p, c->d_r.p);
+        halo_apply_kernel<<<(r1 - r0 + 255) / 256, 256, 0, c->stream>>>(c->d_recv_proc.p, c->d_recvbuf, r0, r1, c->d_colptr.p, c->d_crow.p, c->d_valT.p, c->d_psite.p, c->d_field.p, c->d_r.p);
         launched++;
     }
     return launched;
@@ -879,13 +912,35 @@ static void ensure_zbuf(Ctx *c, size_t count) {
     if (c->d_zbuf.n >= count) return;
     CK(cudaStreamSynchronize(c->stream));
     c->d_zbuf.alloc(count);
-    if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; }  // zbuf pointer is baked in
+    drop_sweep_graph(c);
 }
 
 static void refresh_r(Ctx *c, double beta0) {
     op_spmv(c, c->d_linv[c->cur].p, c->d_field.p, beta0, c->d_r.p);
     c->r_valid = !c->sharded;   // a sharded field's ghost rows are not kept current by its own sweep
     c->r_beta0 = beta0;
+}
+
+// The way into every sweep: commit the current factor if needed, upload the supplied normals (rng_mode NNGP_RNG_SUPPLIED: n_global
+// per sweep, indexed by the position in the whole field), set the sweep parameters and make r current for beta0.
+static void begin_sweeps(Ctx *c, double beta0, double log_scale, double log_noise_variance, int rng_mode, const double *z, int n_sweeps,
+                         double seed) {
+    if (!c->committed) op_commit(c);
+    if (rng_mode == NNGP_RNG_SUPPLIED) {
+        const size_t nz = (size_t)c->n_global * (size_t)std::max(1, n_sweeps);
+        ensure_zbuf(c, nz);
+        CK(cudaMemcpyAsync(c->d_zbuf.p, z, sizeof(double) * nz, cudaMemcpyHostToDevice, c->stream));
+    }
+    set_sweep_params(c, beta0, log_scale, log_noise_variance, rng_mode, seed);
+    refresh_r(c, beta0);
+}
+
+// nngp_time_op / nngp_time_op_group: Philox sweeps under a fixed seed with the scalar parameters of the context's last sweep
+// (set_sweep_params leaves them in h_pinned + 32)
+static void begin_timed_sweeps(Ctx *c) {
+    const SweepParams *sp = reinterpret_cast<SweepParams *>(c->h_pinned + 32);
+    begin_sweeps(c, sp->beta0, -std::log(sp->e_ls > 0 ? sp->e_ls : 1.0), -std::log(sp->e_ln > 0 ? sp->e_ln : 1.0), NNGP_RNG_PHILOX, nullptr, 1,
+                 12345.0);
 }
 
 // ---- dense products with the resident design matrices (update_Gaussian.R:226-246) ----
@@ -978,42 +1033,6 @@ static void flush_l2(Ctx *c) {
     fill_f64_kernel<<<c->n_sm * 8, 256, 0, c->stream>>>(c->d_flush.p, 1.0, c->d_flush.n);
 }
 
-static void destroy_ctx(Ctx *c) {
-    cudaSetDevice(c->device);
-    if (c->stream) cudaStreamSynchronize(c->stream);
-    if (c->sweep_graph) cudaGraphExecDestroy(c->sweep_graph);
-    if (c->comm && g_nccl.ok) g_nccl.CommDestroy(c->comm);
-    for (int h = 0; h < 8; h++) if (c->peer_mapped[h]) cudaIpcCloseMemHandle(c->peer_mapped[h]);
-    c->d_recvbuf.p = nullptr;
-    if (c->p2p_area) cudaFree(c->p2p_area);
-    c->d_shard_state.release(); c->d_bptr.release(); c->d_bdst.release(); c->d_sxptr.release(); c->d_sxdst.release();
-    c->d_ginfo.release(); c->d_shard_tl.release();
-    c->d_send_storage.release(); c->d_recv_proc.release(); c->d_sendbuf.release(); c->d_owned.release();
-    DevBuf<int> *ib[] = {&c->d_psite, &c->d_gid, &c->d_i2g, &c->d_g2i, &c->d_nn, &c->d_colptr, &c->d_crow, &c->d_csrc, &c->d_zpos, &c->d_lvl_rows, &c->d_lvl_ptr,
-                         &c->d_lm, &c->d_optr, &c->d_oidx, &c->d_cstart, &c->d_partial_rows, &c->d_nbad};
-    for (auto *b : ib) b->release();
-    DevBuf<double> *db[] = {&c->d_locs, &c->d_tl, &c->d_linv[0], &c->d_linv[1], &c->d_valT, &c->d_pd, &c->d_nobs, &c->d_ymx, &c->d_S,
-                            &c->d_field, &c->d_newfield, &c->d_r, &c->d_tmp1, &c->d_tmp2, &c->d_io, &c->d_zbuf, &c->d_partials,
-                            &c->d_scalars, &c->d_flush};
-    for (auto *b : db) b->release();
-    c->d_mtab.release();
-    c->d_frec.release();
-    c->d_Xa.release(); c->d_Xl.release(); c->d_B.release(); c->d_yobs.release(); c->d_robs.release(); c->d_coef.release(); c->d_atb_part.release(); c->d_atb_out.release();
-    c->d_pred_rows.release();
-    c->d_sp.release();
-    c->d_tiles.release();
-    c->d_rows_padded.release(); c->d_ticket.release(); c->d_cloc.release();
-    c->d_nn_lvl.release(); c->d_lpos.release(); c->d_linv_lvl[0].release(); c->d_linv_lvl[1].release();
-    if (c->h_pinned) cudaFreeHost(c->h_pinned);
-    if (c->h_stage) cudaFreeHost(c->h_stage);
-    if (c->ev0) cudaEventDestroy(c->ev0);
-    if (c->ev1) cudaEventDestroy(c->ev1);
-    if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-    if (c->ev_copy) cudaEventDestroy(c->ev_copy);
-    if (c->stream) cudaStreamDestroy(c->stream);
-    delete c;
-}
-
 }  // namespace nngp
 
 using namespace nngp;
@@ -1088,7 +1107,6 @@ struct ShardArgs {
 static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const double *locs, const int *NNarray, const int *coloring,
                             const int *n_obs_, const int *locs_match, const int *covfun_id, const int *device, const int *layout,
                             const ShardArgs *sh, int *ctx_id, int *status) {
-    Ctx *c = nullptr;
     ABI_BEGIN
     REQUIRE(n_ && d_ && m_ && locs && NNarray && coloring && n_obs_ && (locs_match || *n_obs_ == 0) && covfun_id && device && layout && ctx_id, "nngp_ctx_create: null argument");
     const int n = *n_, d = *d_, m = *m_, M = m + 1, n_obs = *n_obs_;
@@ -1108,7 +1126,8 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
         std::fprintf(stderr, "[nngp ctx_create] %-28s %8.1f ms\n", what, 1e3 * std::chrono::duration<double>(now - t_create).count());
         t_create = now;
     };
-    c = new Ctx();
+    std::unique_ptr<Ctx> owner(new Ctx());
+    Ctx *c = owner.get();
     c->device = *device;
     c->layout = (*layout == NNGP_LAYOUT_COLOR || *layout == NNGP_LAYOUT_COLOR_MORTON) ? *layout : NNGP_LAYOUT_MORTON;
     c->n = n; c->d = d; c->m = m; c->M = M; c->n_obs = n_obs; c->covfun = *covfun_id;
@@ -1482,8 +1501,7 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
             if (!c->recv_storage.empty())
                 CK(cudaMemcpyAsync(c->p2p_area + c->p2p_tab_off, c->recv_storage.data(), c->recv_storage.size() * sizeof(int), cudaMemcpyHostToDevice, s));
         }
-        c->d_recvbuf.p = c->p2p_area + c->p2p_val_off;      // not owned by the DevBuf (released with the area)
-        c->d_recvbuf.n = 0;
+        c->d_recvbuf = c->p2p_area + c->p2p_val_off;
         ensure_stage(c, (size_t)std::max(n, n_obs));   // no page-locked allocation (a device-synchronising call) once peers may be waiting on this rank
         c->d_shard_state.alloc(4);
         CK(cudaMemsetAsync(c->d_shard_state.p, 0, 4 * sizeof(unsigned long long), s));
@@ -1502,12 +1520,10 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
         int id = -1;
         for (size_t k = 0; k < g_ctx.size(); k++) if (!g_ctx[k]) { id = (int)k; break; }
         if (id < 0) { g_ctx.push_back(nullptr); id = (int)g_ctx.size() - 1; }
-        g_ctx[id] = c;
+        g_ctx[id] = owner.release();
         *ctx_id = id;
     }
-    c = nullptr;
     ABI_END
-    if (c) destroy_ctx(c);
 }
 
 void nngp_ctx_create(const int *n_, const int *d_, const int *m_, const double *locs, const int *NNarray, const int *coloring,
@@ -1541,7 +1557,7 @@ void nngp_ctx_destroy(const int *ctx_id, int *status) {
     ABI_BEGIN
     Ctx *c = get_ctx(ctx_id);
     { std::lock_guard<std::mutex> lk(g_ctx_mu); g_ctx[*ctx_id] = nullptr; }
-    destroy_ctx(c);
+    delete c;
     ABI_END
 }
 
@@ -1562,13 +1578,13 @@ void nngp_ctx_set_option(const int *ctx_id, const int *key, const int *value, in
         case NNGP_OPT_COMMIT_VARIANT: REQUIRE(*value >= 0 && *value <= 1, "commit variant must be 0..1"); c->commit_variant = *value; break;
         case NNGP_OPT_SOLVE_WINDOW_CTAS: REQUIRE(*value >= 0 && *value <= 4096, "solve window must be 0..4096 CTAs"); c->solve_window_ctas = *value; break;
         case NNGP_OPT_SOLVE_LEVEL_COPY: c->level_copy = (*value != 0); c->have_factor[0] = c->have_factor[1] = false; c->committed = false; break;
-        case NNGP_OPT_SHARD_GHOST_CTAS: REQUIRE(*value >= 1 && *value <= 1024, "ghost CTAs must be 1..1024"); c->shard_ghost_ctas = *value; if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; } break;
-        case NNGP_OPT_SHARD_GHOST_FIRST: REQUIRE(*value >= 0 && *value <= 2, "ghost placement must be 0..2"); c->shard_ghost_first = *value; if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; } break;
+        case NNGP_OPT_SHARD_GHOST_CTAS: REQUIRE(*value >= 1 && *value <= 1024, "ghost CTAs must be 1..1024"); c->shard_ghost_ctas = *value; break;
+        case NNGP_OPT_SHARD_GHOST_FIRST: REQUIRE(*value >= 0 && *value <= 2, "ghost placement must be 0..2"); c->shard_ghost_first = *value; break;
         case NNGP_OPT_FACTOR_VARIANT: REQUIRE(*value >= 0 && *value <= 1, "factor variant must be 0..1"); c->factor_variant = *value; break;
         case NNGP_OPT_SOLVE_SLEEP_NS: REQUIRE(*value >= 0 && *value <= 100000, "solve sleep must be 0..100000 ns"); c->solve_sleep_ns = *value; break;
         default: REQUIRE(false, "unknown option key %d", *key);
     }
-    if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; }
+    drop_sweep_graph(c);
     ABI_END
 }
 
@@ -1584,18 +1600,15 @@ void nngp_shard_timeline(const int *ctx_id, const double *beta_0, const double *
     std::vector<unsigned long long> init(cnt);
     for (size_t i = 0; i < cnt; i++) init[i] = (i % 6 == 0 || i % 6 == 2) ? ~0ull : 0ull;   // min-stamps start at +inf
     c->d_shard_tl.upload(init, c->stream);
-    if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; }
+    drop_sweep_graph(c);
     c->shard_tl_on = true;
-    if (!c->committed) op_commit(c);
-    set_sweep_params(c, *beta_0, *log_scale, *log_noise_variance, NNGP_RNG_PHILOX, 1.0);
-    refresh_r(c, *beta_0);
+    begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, NNGP_RNG_PHILOX, nullptr, 1, 1.0);
     op_sweeps(c, 1);
-    c->sweep_counter += 1ull;
     c->shard_tl_on = false;
     std::vector<unsigned long long> t(cnt);
     CK(cudaMemcpyAsync(t.data(), c->d_shard_tl.p, sizeof(unsigned long long) * cnt, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; }
+    drop_sweep_graph(c);
     unsigned long long t0 = ~0ull;
     for (size_t i = 0; i < cnt; i++) if (t[i] != 0ull && t[i] != ~0ull && t[i] < t0) t0 = t[i];
     for (size_t i = 0; i < cnt; i++) out_ns[i] = (t[i] == 0ull || t[i] == ~0ull) ? -1.0 : (double)(t[i] - t0);
@@ -1671,7 +1684,6 @@ void nngp_factor_get(const int *ctx_id, const int *slot, double *Linv, int *stat
     LAUNCHED(c);
     CK(cudaMemcpyAsync(Linv, tmp.p, sizeof(double) * (size_t)c->n * c->M, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    tmp.release();
     ABI_END
 }
 
@@ -1823,16 +1835,8 @@ void nngp_gibbs_sweep(const int *ctx_id, const int *n_sweeps, const double *beta
     NEED(c->have_slot(NNGP_SLOT_CURRENT), "nngp_gibbs_sweep: no current factor");
     NEED(c->have_field && c->have_obs, "nngp_gibbs_sweep: field and observations must be set first");
     use(c);
-    if (!c->committed) op_commit(c);
-    const size_t nz = (size_t)c->n_global * (size_t)std::max(1, *n_sweeps);   // normals are indexed by the position in the whole field
-    if (*rng_mode == NNGP_RNG_SUPPLIED) {
-        ensure_zbuf(c, nz);
-        CK(cudaMemcpyAsync(c->d_zbuf.p, z, sizeof(double) * nz, cudaMemcpyHostToDevice, c->stream));
-    }
-    set_sweep_params(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, seed ? *seed : 0.0);
-    refresh_r(c, *beta_0);
+    begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, z, *n_sweeps, seed ? *seed : 0.0);
     op_sweeps(c, *n_sweeps);
-    c->sweep_counter += (unsigned long long)*n_sweeps;
     CK(cudaStreamSynchronize(c->stream));
     if (c->p2p) check_solve_flag(c);
     ABI_END
@@ -1851,7 +1855,6 @@ void nngp_sweep_loglik_host(const int *ctx_id, const int *n_sweeps, const double
     NEED(c->can_sweep, "this context was created without a colouring (all-zero coloring): it cannot run Gibbs sweeps");
     NEED(c->have_slot(NNGP_SLOT_CURRENT) && c->have_obs, "nngp_sweep_loglik_host: factor and observations must be set first");
     use(c);
-    if (!c->committed) op_commit(c);
     const bool pinned = is_pinned(field_io);
     if (pinned) {   // as upload_site_vector, without its synchronisation: the buffer is not handed back before the download below
         CK(cudaMemcpyAsync(c->d_io.p, field_io, sizeof(double) * c->n, cudaMemcpyHostToDevice, c->stream));
@@ -1861,15 +1864,8 @@ void nngp_sweep_loglik_host(const int *ctx_id, const int *n_sweeps, const double
         upload_site_vector(c, field_io, c->d_field.p);
     }
     c->have_field = true;
-    const size_t nz = (size_t)c->n_global * (size_t)std::max(1, *n_sweeps);
-    if (*rng_mode == NNGP_RNG_SUPPLIED) {
-        ensure_zbuf(c, nz);
-        CK(cudaMemcpyAsync(c->d_zbuf.p, z, sizeof(double) * nz, cudaMemcpyHostToDevice, c->stream));
-    }
-    set_sweep_params(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, seed ? *seed : 0.0);
-    refresh_r(c, *beta_0);
+    begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, z, *n_sweeps, seed ? *seed : 0.0);
     op_sweeps(c, *n_sweeps);
-    c->sweep_counter += (unsigned long long)*n_sweeps;
     if (pinned) {   // the new field leaves on a second stream while the log-lik pass reads it on the first
         gather_f64_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(c->d_io.p, c->d_field.p, c->d_g2i.p, c->n);
         LAUNCHED(c);
@@ -1954,7 +1950,7 @@ static void finish_p2p_connect(Ctx *c, const int *peer_recv_base) {
     // every ghost slot (both parities) starts EMPTY: the value itself is the message (see NNGP_HALO_EMPTY)
     fill_u64_kernel<<<grid_for(c, (long long)(2 * c->p2p_parity_stride), 256), 256, 0, c->stream>>>(reinterpret_cast<unsigned long long *>(c->p2p_area + c->p2p_val_off), NNGP_HALO_EMPTY, (int)(2 * c->p2p_parity_stride));
     CK(cudaStreamSynchronize(c->stream));
-    if (c->sweep_graph) { cudaGraphExecDestroy(c->sweep_graph); c->sweep_graph = nullptr; }
+    drop_sweep_graph(c);
     c->p2p = true;
 }
 
@@ -2034,22 +2030,11 @@ void nngp_shard_group_sweep(const int *ctx_ids, const int *world, const int *n_s
     }
     for (Ctx *c : cs) {
         use(c);
-        if (!c->committed) op_commit(c);
-        const size_t nz = (size_t)c->n_global * (size_t)std::max(1, *n_sweeps);
-        if (*rng_mode == NNGP_RNG_SUPPLIED) {
-            ensure_zbuf(c, nz);
-            CK(cudaMemcpyAsync(c->d_zbuf.p, z, sizeof(double) * nz, cudaMemcpyHostToDevice, c->stream));
-        }
-        set_sweep_params(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, seed ? *seed : 0.0);
-        refresh_r(c, *beta_0);
+        begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, z, *n_sweeps, seed ? *seed : 0.0);
     }
     for (int s = 0; s < *n_sweeps; s++)       // sweep by sweep over the members: no stream runs far ahead of its peers
         for (Ctx *c : cs) { use(c); op_sweeps(c, 1); }
-    for (Ctx *c : cs) {
-        use(c);
-        c->sweep_counter += (unsigned long long)*n_sweeps;
-        CK(cudaStreamSynchronize(c->stream));
-    }
+    for (Ctx *c : cs) { use(c); CK(cudaStreamSynchronize(c->stream)); }
     for (Ctx *c : cs) { use(c); check_solve_flag(c); }
     ABI_END
 }
@@ -2087,13 +2072,7 @@ void nngp_shard_sweep_begin(const int *ctx_id, const double *beta_0, const doubl
     NEED(c->sharded, "nngp_shard_sweep_begin: not a sharded context");
     NEED(c->have_slot(NNGP_SLOT_CURRENT) && c->have_field && c->have_obs, "nngp_shard_sweep_begin: factor, field and observations must be set first");
     use(c);
-    if (!c->committed) op_commit(c);
-    if (*rng_mode == NNGP_RNG_SUPPLIED) {
-        ensure_zbuf(c, (size_t)c->n_global);
-        CK(cudaMemcpyAsync(c->d_zbuf.p, z, sizeof(double) * (size_t)c->n_global, cudaMemcpyHostToDevice, c->stream));
-    }
-    set_sweep_params(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, seed ? *seed : 0.0);
-    refresh_r(c, *beta_0);
+    begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, z, 1, seed ? *seed : 0.0);
     CK(cudaStreamSynchronize(c->stream));
     ABI_END
 }
@@ -2142,8 +2121,8 @@ void nngp_shard_halo_put(const int *ctx_id, const int *colour, const double *in,
     const int r0 = c->recv_ptr[(size_t)col * W], r1 = c->recv_ptr[(size_t)(col + 1) * W];
     if (r1 > r0) {
         REQUIRE(in != nullptr, "nngp_shard_halo_put: null buffer");
-        CK(cudaMemcpyAsync(c->d_recvbuf.p + r0, in, sizeof(double) * (size_t)(r1 - r0), cudaMemcpyHostToDevice, c->stream));
-        halo_apply_kernel<<<(r1 - r0 + 255) / 256, 256, 0, c->stream>>>(c->d_recv_proc.p, c->d_recvbuf.p, r0, r1, c->d_colptr.p, c->d_crow.p, c->d_valT.p, c->d_psite.p, c->d_field.p, c->d_r.p);
+        CK(cudaMemcpyAsync(c->d_recvbuf + r0, in, sizeof(double) * (size_t)(r1 - r0), cudaMemcpyHostToDevice, c->stream));
+        halo_apply_kernel<<<(r1 - r0 + 255) / 256, 256, 0, c->stream>>>(c->d_recv_proc.p, c->d_recvbuf, r0, r1, c->d_colptr.p, c->d_crow.p, c->d_valT.p, c->d_psite.p, c->d_field.p, c->d_r.p);
         LAUNCHED(c);
     }
     CK(cudaStreamSynchronize(c->stream));
@@ -2549,15 +2528,11 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         // ---- (D) chromatic sweeps :257-275 ----
         nvtxRangePushA("nngp D chromatic Gibbs sweeps");
         if (rng_mode == NNGP_RNG_SUPPLIED) {
-            ensure_zbuf(c, (size_t)nz * std::max(1, n_chromatic));
             zhost.resize((size_t)nz * std::max(1, n_chromatic));
             rs.rnorm(zhost.data(), (int64_t)nz * n_chromatic);
-            CK(cudaMemcpyAsync(c->d_zbuf.p, zhost.data(), sizeof(double) * (size_t)nz * n_chromatic, cudaMemcpyHostToDevice, c->stream));
         }
-        set_sweep_params(c, beta_0, log_scale, lnv, rng_mode, (double)philox_seed);
-        refresh_r(c, beta_0);
+        begin_sweeps(c, beta_0, log_scale, lnv, rng_mode, zhost.data(), n_chromatic, (double)philox_seed);   // zbuf sized by prepare_chain_buffers
         op_sweeps(c, n_chromatic);
-        c->sweep_counter += (unsigned long long)n_chromatic;
         mark(3);
         nvtxRangePop();
         // ---- (E) noise variance :281-293 ----
@@ -2710,6 +2685,17 @@ struct ChainJob {
     std::string error;
 };
 
+// a worker's status turned back into the exception that set it (the message is already set)
+[[noreturn]] static void throw_status(int status) {
+    switch (status) {
+        case NNGP_ERR_CUDA: throw CudaFail();
+        case NNGP_ERR_STATE: throw StateFail();
+        case NNGP_ERR_NCCL: throw NcclFail();
+        case NNGP_ERR_ALLOC: throw std::bad_alloc();
+        default: throw ArgFail();
+    }
+}
+
 static void run_chain_jobs(std::vector<ChainJob> &jobs, int max_concurrent, const int *n_shape, const int *n_iter, const double *thin,
                            const int *n_chromatic, const int *iter_start, const int *rng_mode, const double *var_y,
                            const double *solve_1XT1X, const double *chol_1XT1X) {
@@ -2776,13 +2762,7 @@ static void chains_run_common(const int *n_chains_, const int *ctx_ids, const in
     for (int k = 0; k < nc; k++)
         if (jobs[k].status != NNGP_OK) {
             set_error("chain %d: %s", k + 1, jobs[k].error.c_str());
-            switch (jobs[k].status) {
-                case NNGP_ERR_CUDA: throw CudaFail();
-                case NNGP_ERR_STATE: throw StateFail();
-                case NNGP_ERR_NCCL: throw NcclFail();
-                case NNGP_ERR_ALLOC: throw std::bad_alloc();
-                default: throw ArgFail();
-            }
+            throw_status(jobs[k].status);
         }
     ABI_END
 }
@@ -2844,13 +2824,7 @@ void nngp_shard_group_chain_run(const int *ctx_ids, const int *world, const int 
     for (int h = 0; h < W; h++)
         if (jobs[h].status != NNGP_OK) {
             set_error("member %d: %s", h, jobs[h].error.c_str());
-            switch (jobs[h].status) {
-                case NNGP_ERR_CUDA: throw CudaFail();
-                case NNGP_ERR_STATE: throw StateFail();
-                case NNGP_ERR_NCCL: throw NcclFail();
-                case NNGP_ERR_ALLOC: throw std::bad_alloc();
-                default: throw ArgFail();
-            }
+            throw_status(jobs[h].status);
         }
     for (int h = 1; h < W; h++) {
         REQUIRE(p[h] == p[0] && rec[h] == rec[0] && acc[h] == acc[0], "nngp_shard_group_chain_run: member %d fell out of step with member 0 (their scalar records differ)", h);
@@ -2877,7 +2851,6 @@ void nngp_records_summary(const int *ctx_id, const int *first_row, const int *n_
     LAUNCHED(c);
     CK(cudaMemcpyAsync(out, dout.p, sizeof(double) * (size_t)n * 5, cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    scratch.release(); dout.release(); doff.release();
     ABI_END
 }
 
@@ -2894,9 +2867,7 @@ void nngp_time_op(const int *ctx_id, const int *op_, const int *reps_, const int
     if (op == 2 || op == 6) {
         NEED(c->can_sweep, "this context was created without a colouring (all-zero coloring): it cannot run Gibbs sweeps");
         NEED(c->have_field && c->have_obs, "nngp_time_op(sweep): field and observations must be set first");
-        const SweepParams *sp = reinterpret_cast<SweepParams *>(c->h_pinned + 32);
-        set_sweep_params(c, sp->beta0, -std::log(sp->e_ls > 0 ? sp->e_ls : 1.0), -std::log(sp->e_ln > 0 ? sp->e_ln : 1.0), NNGP_RNG_PHILOX, 12345.0);
-        refresh_r(c, sp->beta0);
+        begin_timed_sweeps(c);
     }
     if (op == 1 || op == 3 || op == 4 || op == 6) NEED(c->have_field, "nngp_time_op: field must be set first");
     CK(cudaStreamSynchronize(c->stream));
@@ -2907,12 +2878,12 @@ void nngp_time_op(const int *ctx_id, const int *op_, const int *reps_, const int
         switch (op) {
             case 0: op_factor_build(c, NNGP_SLOT_PROPOSAL, c->last_cc); break;
             case 1: op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, false); break;
-            case 2: op_sweeps(c, 1); c->sweep_counter++; break;
+            case 2: op_sweeps(c, 1); break;
             case 3: op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, c->d_tmp1.p); break;
             case 4: op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, c->d_tmp1.p);
                     op_sptrsv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_tmp1.p, c->d_tmp2.p, nullptr, 0.0, 1.0); break;
             case 5: op_commit(c); break;
-            case 6: op_sweeps(c, 1); c->sweep_counter++;
+            case 6: op_sweeps(c, 1);
                     op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, true); break;
             default: REQUIRE(false, "nngp_time_op: unknown op %d", op);
         }
@@ -2943,12 +2914,8 @@ void nngp_time_op_group(const int *ctx_ids, const int *n_ctx, const int *op_, co
     }
     use(cs[0]);
     for (Ctx *c : cs) {
-        if (!c->committed) op_commit(c);
-        const SweepParams *sp = reinterpret_cast<SweepParams *>(c->h_pinned + 32);
-        set_sweep_params(c, sp->beta0, -std::log(sp->e_ls > 0 ? sp->e_ls : 1.0), -std::log(sp->e_ln > 0 ? sp->e_ln : 1.0), NNGP_RNG_PHILOX, 12345.0);
-        refresh_r(c, sp->beta0);
+        begin_timed_sweeps(c);
         op_sweeps(c, 1);   // instantiates the graph outside the timed region
-        c->sweep_counter++;
         CK(cudaStreamSynchronize(c->stream));
     }
     // a common origin: every stream waits for one event recorded on the first stream
@@ -2957,7 +2924,6 @@ void nngp_time_op_group(const int *ctx_ids, const int *n_ctx, const int *op_, co
     for (int r = 0; r < *reps_; r++)
         for (Ctx *c : cs) {
             op_sweeps(c, 1);
-            c->sweep_counter++;
             if (*op_ == 6) op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, true);
         }
     for (Ctx *c : cs) CK(cudaEventRecord(c->ev1, c->stream));
@@ -2982,27 +2948,27 @@ void nngp_fp64_peak(const int *device, double *gflops, int *status) {
     CK(cudaSetDevice(*device));
     cudaDeviceProp prop;
     CK(cudaGetDeviceProperties(&prop, *device));
-    double *d_out = nullptr;
-    CK(cudaMalloc(&d_out, sizeof(double)));
-    cudaEvent_t e0, e1;
-    CK(cudaEventCreate(&e0));
-    CK(cudaEventCreate(&e1));
+    DevBuf<double> d_out;
+    d_out.alloc(1);
+    struct Events {
+        cudaEvent_t e0 = nullptr, e1 = nullptr;
+        ~Events() { if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); }
+    } ev;
+    CK(cudaEventCreate(&ev.e0));
+    CK(cudaEventCreate(&ev.e1));
     const int blocks = prop.multiProcessorCount * 8, iters = 4096;
     double best = 0.0;
     for (int rep = 0; rep < 6; rep++) {
-        CK(cudaEventRecord(e0, 0));
-        fp64_peak_kernel<<<blocks, 256>>>(d_out, iters, 1.0000001, 1e-9);
-        CK(cudaEventRecord(e1, 0));
-        CK(cudaEventSynchronize(e1));
+        CK(cudaEventRecord(ev.e0, 0));
+        fp64_peak_kernel<<<blocks, 256>>>(d_out.p, iters, 1.0000001, 1e-9);
+        CK(cudaEventRecord(ev.e1, 0));
+        CK(cudaEventSynchronize(ev.e1));
         float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, e0, e1));
+        CK(cudaEventElapsedTime(&ms, ev.e0, ev.e1));
         g_launches.fetch_add(1, std::memory_order_relaxed);
         const double flops = (double)blocks * 256.0 * iters * 64.0 * 2.0;
         if (rep > 0) best = std::max(best, flops / (ms * 1e-3) / 1e9);
     }
-    cudaEventDestroy(e0);
-    cudaEventDestroy(e1);
-    cudaFree(d_out);
     *gflops = best;
     ABI_END
 }
