@@ -267,6 +267,8 @@ struct Ctx {
     bool matern_table = true;              // tabulate the Matern kernel per factor build (false: evaluate K_nu per pair)
     DevBuf<double> d_locs, d_tl, d_linv[2], d_valT, d_pd, d_nobs, d_ymx, d_S, d_field, d_newfield, d_r, d_tmp1, d_tmp2, d_io,
         d_zbuf, d_partials, d_scalars, d_flush;
+    DevBuf<double> d_logdet;               // sum log linv[cur][0,q] when logdet_valid (filled by the first log-lik from the residual)
+    bool logdet_valid = false;             // cleared by op_commit, where a factor becomes the sweep's
     DevBuf<SweepParams> d_sp;
     DevBuf<int> d_send_storage, d_recv_proc;
     DevBuf<int4> d_ginfo;
@@ -309,7 +311,8 @@ struct Ctx {
     CovConst last_cc{};
     bool have_cc = false;
     unsigned long long sweep_counter = 0;
-    cudaGraphExec_t sweep_graph = nullptr;
+    cudaGraphExec_t sweep_graph = nullptr;   // one sweep, closed by advance_sweep_kernel
+    cudaGraphExec_t step_graph = nullptr;    // one sweep, closed by the log-lik from its residual (loglik_residual_kernel)
     bool use_graph = true;
 
     double *linv_slot(int slot) { return d_linv[slot == NNGP_SLOT_CURRENT ? cur : 1 - cur].p; }
@@ -317,10 +320,11 @@ struct Ctx {
     ~Ctx();
 };
 
-// the captured sweep bakes in buffer pointers and options: dropped whenever one of them changes
+// the captured sweeps bake in buffer pointers and options: dropped whenever one of them changes
 static void drop_sweep_graph(Ctx *c) {
     if (c->sweep_graph) cudaGraphExecDestroy(c->sweep_graph);
-    c->sweep_graph = nullptr;
+    if (c->step_graph) cudaGraphExecDestroy(c->step_graph);
+    c->sweep_graph = c->step_graph = nullptr;
 }
 
 // the teardown whose order matters; the DevBuf members free themselves after it
@@ -570,15 +574,42 @@ static bool launch_loglik_tma(Ctx *c, const double *linv, const double *field, d
     return true;
 }
 
-// partial sums -> d_scalars[off..off+1].  allow_residual: the caller accepts the sums taken from the sweep's residual when it is
-// current for exactly this factor, field and beta_0 (an unsharded context); they differ from the full pass by the rounding the
-// sweep's incremental updates of r accumulated
+// the sums of the log-lik of (linv, field, shift) may be taken from the sweep's residual: it is current for exactly this factor,
+// field and beta_0 (an unsharded context).  They differ from the full pass by the rounding the sweep's incremental updates of r
+// accumulated.
+static bool residual_current(Ctx *c, const double *linv, const double *field, double shift) {
+    return c->loglik_from_residual && !c->sharded && c->r_valid && linv == c->d_linv[c->cur].p && field == c->d_field.p &&
+           std::memcmp(&shift, &c->r_beta0, sizeof(double)) == 0;
+}
+
+// the log-determinant term of the current factor in d_logdet, computed once per factor op_commit makes current
+static void ensure_logdet(Ctx *c) {
+    if (c->logdet_valid) return;
+    logdet_kernel<<<std::min(kReduceBlocks, (c->n + 255) / 256), 256, 0, c->stream>>>(
+        c->d_linv[c->cur].p, c->n, c->d_partials.p, reinterpret_cast<unsigned int *>(c->d_ticket.p + 1), c->d_logdet.p);
+    LAUNCHED(c);
+    c->logdet_valid = true;
+}
+
+// loglik_residual_kernel -> d_scalars[0..1]; spp: the kernel also closes the sweep it follows
+static void launch_loglik_residual(Ctx *c, const cudaLaunchConfig_t &lc, SweepParams *spp) {
+    cudaLaunchConfig_t l = lc;
+    l.gridDim = dim3(std::min(kReduceBlocks, (c->n + 255) / 256));
+    l.blockDim = dim3(256);
+    CK(cudaLaunchKernelEx(&l, loglik_residual_kernel, (const double *)c->d_r.p, c->n, (const double *)c->d_logdet.p, c->d_partials.p,
+                          reinterpret_cast<unsigned int *>(c->d_ticket.p + 1), spp, (unsigned long long)c->n_global, c->d_scalars.p));
+}
+
+// partial sums -> d_scalars[off..off+1].  allow_residual: the caller accepts the sums taken from the sweep's residual when
+// residual_current holds (they go to d_scalars[0..1], where the step graph writes them)
 static void op_loglik_sums(Ctx *c, const double *linv, const double *field, double shift, int scal_off, bool allow_residual) {
     int blocks = std::min(kReduceBlocks, (c->n + 255) / 256);
-    if (allow_residual && c->loglik_from_residual && !c->sharded && c->r_valid && linv == c->d_linv[c->cur].p && field == c->d_field.p &&
-        std::memcmp(&shift, &c->r_beta0, sizeof(double)) == 0) {
-        loglik_residual_kernel<<<blocks, 256, 0, c->stream>>>(linv, c->d_r.p, c->n, reinterpret_cast<double2 *>(c->d_partials.p),
-                                                              reinterpret_cast<unsigned int *>(c->d_ticket.p + 1), c->d_scalars.p + scal_off);
+    if (allow_residual && residual_current(c, linv, field, shift)) {
+        REQUIRE(scal_off == 0, "internal: the log-lik from the residual writes d_scalars[0..1], not [%d..%d]", scal_off, scal_off + 1);
+        ensure_logdet(c);
+        cudaLaunchConfig_t lc = {};
+        lc.stream = c->stream;
+        launch_loglik_residual(c, lc, nullptr);
         LAUNCHED(c);
         return;
     }
@@ -685,6 +716,7 @@ static void op_commit(Ctx *c) {
         LAUNCHED(c);
     }
     c->committed = true;
+    c->logdet_valid = false;
 }
 
 static ShardConst shard_const(Ctx *c) {
@@ -705,8 +737,9 @@ static ShardConst shard_const(Ctx *c) {
 // One launch per colour.  Unsharded field or a sharded one with the peer-to-peer transport: a chain of programmatic
 // dependent launches (colour c+1's r-independent prologue overlaps colour c); with the peer-to-peer transport the same kernel
 // also pushes the boundary values to the peers and applies the ghost values that arrive (gibbs_tile2_kernel<.., SHARD>).
-// Returns the number of kernels launched.
-static int launch_sweep_colors(Ctx *c) {
+// One more launch closes the sweep: advance_sweep_kernel, or with_loglik the log-lik from the residual (residual_current must hold
+// and d_logdet be filled).  Returns the number of kernels launched.
+static int launch_sweep_colors(Ctx *c, bool with_loglik) {
     const bool fused_halo = c->sharded && c->p2p && c->world > 1;
     const ShardConst sc = fused_halo ? shard_const(c) : ShardConst{};
     int launched = 0;
@@ -770,37 +803,68 @@ static int launch_sweep_colors(Ctx *c) {
         launched++;
         if (c->sharded && !fused_halo) launched += op_halo_exchange(c, col);
     }
-    advance_sweep_kernel<<<1, 32, 0, c->stream>>>(c->d_sp.p, (unsigned long long)c->n_global, fused_halo ? c->d_shard_state.p : nullptr);
+    // unsharded PDL chain: the closing kernel is a programmatic dependent of the last colour, resident when that colour completes
+    // instead of launched after it; it waits before it reads or writes anything
+    cudaLaunchConfig_t lc = {};
+    lc.stream = c->stream;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
+    lc.attrs = at;
+    lc.numAttrs = (!c->sharded && c->sweep_variant != 2 && c->sweep_variant != 3 && launched > 0) ? 1 : 0;
+    if (with_loglik) {
+        launch_loglik_residual(c, lc, c->d_sp.p);
+    } else {
+        lc.gridDim = dim3(1);
+        lc.blockDim = dim3(32);
+        CK(cudaLaunchKernelEx(&lc, advance_sweep_kernel, c->d_sp.p, (unsigned long long)c->n_global, fused_halo ? c->d_shard_state.p : nullptr));
+    }
     return launched + 1;
 }
 
-// n_sweeps sweeps over all colours; scalar parameters are read from d_sp.  Nothing in the sequence depends on host-side values
-// (the NCCL transport excepted), so one sweep is captured once and replayed as a CUDA graph: K + 1 plain launches per sweep were
-// CPU-submission bound.  The host's sweep counter advances with every sweep enqueued, as d_sp's does when it runs.
-static void op_sweeps(Ctx *c, int n_sweeps) {
-    if (n_sweeps <= 0) return;
-    const bool graphable = c->use_graph && !(c->sharded && c->world > 1 && !c->p2p);
-    for (int s = 0; s < n_sweeps; s++) {
-        int nl;
-        if (graphable) {
-            if (!c->sweep_graph) {
-                cudaGraph_t g;
-                CK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
-                c->graph_launches = launch_sweep_colors(c);
-                CK(cudaStreamEndCapture(c->stream, &g));
-                CK(cudaGraphInstantiate(&c->sweep_graph, g, 0));
-                CK(cudaGraphDestroy(g));
-            }
-            CK(cudaGraphLaunch(c->sweep_graph, c->stream));
-            nl = c->graph_launches;
-        } else {
-            nl = launch_sweep_colors(c);
-            CK(cudaGetLastError());
+// One sweep over all colours; scalar parameters are read from d_sp.  Nothing in the sequence depends on host-side values (the
+// NCCL transport excepted), so each form of the sweep (see launch_sweep_colors) is captured once and replayed as a CUDA graph: K + 1
+// plain launches per sweep were CPU-submission bound.  The host's sweep counter advances with every sweep enqueued, as d_sp's does
+// when it runs.
+static void op_sweep(Ctx *c, bool with_loglik) {
+    int nl;
+    if (c->use_graph && !(c->sharded && c->world > 1 && !c->p2p)) {
+        cudaGraphExec_t &ge = with_loglik ? c->step_graph : c->sweep_graph;
+        if (!ge) {
+            cudaGraph_t g;
+            CK(cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal));
+            c->graph_launches = launch_sweep_colors(c, with_loglik);   // the same count for both forms
+            CK(cudaStreamEndCapture(c->stream, &g));
+            CK(cudaGraphInstantiate(&ge, g, 0));
+            CK(cudaGraphDestroy(g));
         }
-        g_launches.fetch_add(nl, std::memory_order_relaxed);
-        c->launches_in_op += nl;
-        c->sweep_counter++;
+        CK(cudaGraphLaunch(ge, c->stream));
+        nl = c->graph_launches;
+    } else {
+        nl = launch_sweep_colors(c, with_loglik);
+        CK(cudaGetLastError());
     }
+    g_launches.fetch_add(nl, std::memory_order_relaxed);
+    c->launches_in_op += nl;
+    c->sweep_counter++;
+}
+
+static void op_sweeps(Ctx *c, int n_sweeps) {
+    for (int s = 0; s < n_sweeps; s++) op_sweep(c, false);
+}
+
+// n_sweeps sweeps, then the log-lik sums of the current factor and the field at beta_0 = shift -> d_scalars[0..1].  Where the sums
+// come from the sweep's residual, the last sweep is closed by the log-lik kernel itself (one chain of launches for the step); with
+// n_sweeps = 0 the log-lik is a launch of its own that leaves the sweep counter alone.
+static void op_sweeps_loglik(Ctx *c, int n_sweeps, double shift) {
+    if (n_sweeps > 0 && residual_current(c, c->d_linv[c->cur].p, c->d_field.p, shift)) {
+        ensure_logdet(c);
+        op_sweeps(c, n_sweeps - 1);
+        op_sweep(c, true);
+        return;
+    }
+    op_sweeps(c, n_sweeps);
+    op_loglik_sums(c, c->d_linv[c->cur].p, c->d_field.p, shift, 0, true);
 }
 
 static void set_sweep_params(Ctx *c, double beta0, double log_scale, double log_noise_variance, int rng_mode, double seed) {
@@ -1418,7 +1482,7 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
     if (!c->partial_rows.empty()) c->d_partial_rows.upload(c->partial_rows, s);
     c->d_nbad.alloc(8);   // [0] rows with a non-PD block, [1] wait timed out (1 solve, 2 halo / reduction), [3..5] which solve row waited for what
     CK(cudaMemsetAsync(c->d_nbad.p, 0, 8 * sizeof(int), s));
-    c->d_ticket.alloc(2);   // [0] the triangular solve's chunk tickets, [1] the residual log-lik's CTA count (back to 0 after every launch)
+    c->d_ticket.alloc(2);   // [0] the triangular solve's chunk tickets, [1] last_cta_sum's CTA count (back to 0 after every launch)
     CK(cudaMemsetAsync(c->d_ticket.p, 0, 2 * sizeof(int), s));
     c->d_rows_padded.upload(rows_padded, s);
     {   // level-ordered copies for the triangular solve: static neighbour table now, factor values at every factor build
@@ -1445,7 +1509,7 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
     CK(cudaMemsetAsync(c->d_valT.p + c->nnz, 0, 2 * sizeof(double), s));
     c->d_pd.alloc(n); c->d_ymx.alloc(std::max(n_obs, 1)); c->d_S.alloc(n); c->d_field.alloc(n);
     c->d_newfield.alloc(n); c->d_r.alloc(n); c->d_tmp1.alloc(n); c->d_tmp2.alloc(n); c->d_io.alloc((size_t)std::max(n, n_obs));
-    c->d_zbuf.alloc(n); c->d_partials.alloc((size_t)kReduceBlocks * 4); c->d_scalars.alloc(64); c->d_sp.alloc(1);
+    c->d_zbuf.alloc(n); c->d_partials.alloc((size_t)kReduceBlocks * 4); c->d_scalars.alloc(64); c->d_logdet.alloc(1); c->d_sp.alloc(1);
     CK(cudaMemsetAsync(c->d_S.p, 0, sizeof(double) * n, s));
     if (sh) {
         const int W = sh->world;
@@ -1865,8 +1929,10 @@ void nngp_sweep_loglik_host(const int *ctx_id, const int *n_sweeps, const double
     }
     c->have_field = true;
     begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, z, *n_sweeps, seed ? *seed : 0.0);
-    op_sweeps(c, *n_sweeps);
-    if (pinned) {   // the new field leaves on a second stream while the log-lik pass reads it on the first
+    if (pinned) {
+        // the new field leaves on a second stream while the log-lik (from r, or the full pass) runs on the first.  Closing the last
+        // sweep with the log-lik instead (op_sweeps_loglik) makes the copy wait for it: 0.6 % slower end to end (profiles/r04_step_tail.txt)
+        op_sweeps(c, *n_sweeps);
         gather_f64_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(c->d_io.p, c->d_field.p, c->d_g2i.p, c->n);
         LAUNCHED(c);
         CK(cudaEventRecord(c->ev_copy, c->stream));
@@ -1877,7 +1943,7 @@ void nngp_sweep_loglik_host(const int *ctx_id, const int *n_sweeps, const double
         CK(cudaStreamSynchronize(c->stream));
         CK(cudaStreamSynchronize(c->copy_stream));
     } else {
-        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, 0, true);
+        op_sweeps_loglik(c, *n_sweeps, *beta_0);
         CK(cudaMemcpyAsync(c->h_pinned, c->d_scalars.p, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
         download_site_vector(c, c->d_field.p, field_io);   // synchronises
     }
@@ -2868,6 +2934,8 @@ void nngp_time_op(const int *ctx_id, const int *op_, const int *reps_, const int
         NEED(c->can_sweep, "this context was created without a colouring (all-zero coloring): it cannot run Gibbs sweeps");
         NEED(c->have_field && c->have_obs, "nngp_time_op(sweep): field and observations must be set first");
         begin_timed_sweeps(c);
+        // a new factor's log-determinant term is computed here, not inside the first timed step
+        if (op == 6 && residual_current(c, c->d_linv[c->cur].p, c->d_field.p, 0.0)) ensure_logdet(c);
     }
     if (op == 1 || op == 3 || op == 4 || op == 6) NEED(c->have_field, "nngp_time_op: field must be set first");
     CK(cudaStreamSynchronize(c->stream));
@@ -2883,8 +2951,7 @@ void nngp_time_op(const int *ctx_id, const int *op_, const int *reps_, const int
             case 4: op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, c->d_tmp1.p);
                     op_sptrsv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_tmp1.p, c->d_tmp2.p, nullptr, 0.0, 1.0); break;
             case 5: op_commit(c); break;
-            case 6: op_sweeps(c, 1);
-                    op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, true); break;
+            case 6: op_sweeps_loglik(c, 1, 0.0); break;
             default: REQUIRE(false, "nngp_time_op: unknown op %d", op);
         }
         CK(cudaEventRecord(c->ev1, c->stream));
@@ -2915,7 +2982,8 @@ void nngp_time_op_group(const int *ctx_ids, const int *n_ctx, const int *op_, co
     use(cs[0]);
     for (Ctx *c : cs) {
         begin_timed_sweeps(c);
-        op_sweeps(c, 1);   // instantiates the graph outside the timed region
+        if (*op_ == 6) op_sweeps_loglik(c, 1, 0.0);   // instantiates the graph outside the timed region
+        else op_sweeps(c, 1);
         CK(cudaStreamSynchronize(c->stream));
     }
     // a common origin: every stream waits for one event recorded on the first stream
@@ -2923,8 +2991,8 @@ void nngp_time_op_group(const int *ctx_ids, const int *n_ctx, const int *op_, co
     for (int k = 1; k < nc; k++) CK(cudaStreamWaitEvent(cs[k]->stream, cs[0]->ev0, 0));
     for (int r = 0; r < *reps_; r++)
         for (Ctx *c : cs) {
-            op_sweeps(c, 1);
-            if (*op_ == 6) op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, 0.0, 0, true);
+            if (*op_ == 6) op_sweeps_loglik(c, 1, 0.0);
+            else op_sweeps(c, 1);
         }
     for (Ctx *c : cs) CK(cudaEventRecord(c->ev1, c->stream));
     double worst = 0.0;
