@@ -182,6 +182,26 @@ struct DevBuf {
     }
 };
 
+// Slots of d_scalars: a reduction's two sums go to pair A or B; the chain's all-reduced host values and the solve barrier have their own
+enum ScalarSlot : int { kPairA = 0, kPairB = 2, kNObsSlot = 16, kNotPdSlot = 17, kBarrierSlot = 60, kScalarSlots = 64 };
+// Words of d_nbad, the device status: rows whose block was not positive definite (the factor builds count them); the wait flag
+// (1 = solve, 2 = halo or reduction), which kernels get as `err`; the row, site and chunk of a sharded solve's wait (err[2..4]).
+enum StatusWord : int { kNotPd = 0, kWaitFlag = 1, kSolveWaitRow = 3, kSolveWaitSite = 4, kSolveWaitChunk = 5, kStatusWords = 8 };
+// Words of d_ticket: the sync-free solve's chunk ticket; last_cta_sum's CTA count (back to 0 after every launch)
+enum TicketWord : int { kSolveTicket = 0, kCtaCount = 1, kTicketWords = 2 };
+// Words of d_shard_state: sweeps completed since the peers were connected; (colour, ghost slot, sweep) of a halo wait that timed out
+enum ShardStateWord : int { kSweepsSinceConnect = 0, kHaloWaitColour = 1, kHaloWaitSlot = 2, kHaloWaitSweep = 3, kShardStateWords = 4 };
+
+// The pinned host side of the scalars that cross PCIe, one allocation.  sp is the source of an asynchronous upload: set_sweep_params
+// rewrites it only after the stream has consumed the previous copy (the stream is synchronised between any two of its calls).
+struct HostScalars {
+    double sums[kPairB + 2];         // fetch_scalars: pairs A and B of d_scalars, at their slots
+    int status[kStatusWords];        // read_status: a copy of d_nbad
+    double n_obs_sum, not_pd_sum;    // the chain's host values, summed over the ranks of a sharded field
+    SweepParams sp;                  // staged by set_sweep_params
+    unsigned long long area_hdr[5];  // header of the peer-to-peer area (create_ctx_impl)
+};
+
 struct Ctx {
     int device = 0, layout = NNGP_LAYOUT_MORTON;
     cudaStream_t stream = nullptr;
@@ -208,7 +228,7 @@ struct Ctx {
     std::vector<int> send_proc;            // processing id of every entry of the send lists
     std::vector<int> send_storage_h;       // storage id of the same
     std::vector<int> btile_count;          // per colour: tiles that hold boundary sites (they come first inside the colour)
-    DevBuf<unsigned long long> d_shard_state;         // [0] sweeps since connect, [1 + colour] boundary tiles done
+    DevBuf<unsigned long long> d_shard_state;         // ShardStateWord: sweeps since connect, the last halo wait that timed out
     DevBuf<int> d_bptr;
     DevBuf<int2> d_bdst;
     long long nnz = 0;
@@ -286,7 +306,7 @@ struct Ctx {
     int factor_variant = 0;                // 0 = thread per row everywhere (default), 1 = warp-per-row kernel where it exists (m = 20)
     DevBuf<unsigned long long> d_solve_tl;   // development aid: per-chunk completion times of the sync-free solve
     bool solve_tl_on = false;
-    double *h_pinned = nullptr;       // 64 doubles of pinned scratch for scalar results
+    HostScalars *hs = nullptr;
     double *h_stage = nullptr;        // pinned staging for vectors (n doubles at least)
     size_t h_stage_n = 0;
 
@@ -311,6 +331,7 @@ struct Ctx {
     CovConst last_cc{};
     bool have_cc = false;
     unsigned long long sweep_counter = 0;
+    double sweep_beta0 = 0.0, sweep_log_scale = 0.0, sweep_log_noise_variance = 0.0;   // of the last sweep (set_sweep_params)
     cudaGraphExec_t sweep_graph = nullptr;   // one sweep, closed by advance_sweep_kernel
     cudaGraphExec_t step_graph = nullptr;    // one sweep, closed by the log-lik from its residual (loglik_residual_kernel)
     bool use_graph = true;
@@ -335,7 +356,7 @@ Ctx::~Ctx() {
     if (comm && g_nccl.ok) g_nccl.CommDestroy(comm);
     for (int h = 0; h < 8; h++) if (peer_mapped[h]) cudaIpcCloseMemHandle(peer_mapped[h]);
     if (p2p_area) cudaFree(p2p_area);
-    if (h_pinned) cudaFreeHost(h_pinned);
+    if (hs) cudaFreeHost(hs);
     if (h_stage) cudaFreeHost(h_stage);
     if (ev0) cudaEventDestroy(ev0);
     if (ev1) cudaEventDestroy(ev1);
@@ -483,7 +504,7 @@ static void launch_factor(Ctx *c, double *linv, const CovConst &cc) {
     const int blk = 128, grd = (n + blk - 1) / blk;
 #define FACTOR_CASE(MM, DD)                                                                                              \
     if (!specialised && M == MM && c->dt == DD) {                                                                                        \
-        vecchia_factor_reg_kernel<MM, DD, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p); \
+        vecchia_factor_reg_kernel<MM, DD, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p + kNotPd); \
         specialised = true;                                                                                              \
     }
     FACTOR_CASE(6, 2)
@@ -495,16 +516,16 @@ static void launch_factor(Ctx *c, double *linv, const CovConst &cc) {
         const int blocks = std::max(1, std::min((n + 31) / 32, c->n_sm * 2));
         if (c->dt == 2) {
             CK(cudaFuncSetAttribute(vecchia_factor_warp_kernel<21, 2, MATERN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            vecchia_factor_warp_kernel<21, 2, MATERN><<<blocks, 256, smem, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p);
+            vecchia_factor_warp_kernel<21, 2, MATERN><<<blocks, 256, smem, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p + kNotPd);
         } else {
             CK(cudaFuncSetAttribute(vecchia_factor_warp_kernel<21, 3, MATERN>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            vecchia_factor_warp_kernel<21, 3, MATERN><<<blocks, 256, smem, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p);
+            vecchia_factor_warp_kernel<21, 3, MATERN><<<blocks, 256, smem, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p + kNotPd);
         }
         LAUNCHED(c);
         return;
     }
     if (!specialised && M == 21 && c->dt == 2) {   // thread per row, 231-entry triangle: all 255 registers and spills to L1 beyond (comparison)
-        vecchia_factor_reg_kernel<21, 2, MATERN, 1><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p);
+        vecchia_factor_reg_kernel<21, 2, MATERN, 1><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, n, ld, cc, c->d_nbad.p + kNotPd);
         specialised = true;
     }
 #undef FACTOR_CASE
@@ -512,15 +533,15 @@ static void launch_factor(Ctx *c, double *linv, const CovConst &cc) {
         LAUNCHED(c);
         const int np = M <= 24 ? 0 : (int)c->partial_rows.size();   // partial rows ride along in the main launch
         if (np > 0) {
-            vecchia_factor_generic_kernel<24, MATERN><<<(np + blk - 1) / blk, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, c->d_partial_rows.p, np, ld, M, cc, c->d_nbad.p);
+            vecchia_factor_generic_kernel<24, MATERN><<<(np + blk - 1) / blk, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, c->d_partial_rows.p, np, ld, M, cc, c->d_nbad.p + kNotPd);
             LAUNCHED(c);
         }
         return;
     }
-    if (M <= 8) vecchia_factor_generic_kernel<8, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p);
-    else if (M <= 16) vecchia_factor_generic_kernel<16, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p);
-    else if (M <= 24) vecchia_factor_generic_kernel<24, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p);
-    else vecchia_factor_generic_kernel<32, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p);
+    if (M <= 8) vecchia_factor_generic_kernel<8, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p + kNotPd);
+    else if (M <= 16) vecchia_factor_generic_kernel<16, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p + kNotPd);
+    else if (M <= 24) vecchia_factor_generic_kernel<24, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p + kNotPd);
+    else vecchia_factor_generic_kernel<32, MATERN><<<grd, blk, 0, c->stream>>>(c->d_nn.p, c->d_tl.p, linv, nullptr, n, ld, M, cc, c->d_nbad.p + kNotPd);
     LAUNCHED(c);
 }
 
@@ -533,7 +554,7 @@ static void op_factor_build(Ctx *c, int slot, const CovConst &cc_in) {
         LAUNCHED(c);
         cc.mtab = c->d_mtab.p;
     }
-    CK(cudaMemsetAsync(c->d_nbad.p, 0, 2 * sizeof(int), c->stream));
+    CK(cudaMemsetAsync(c->d_nbad.p + kNotPd, 0, 2 * sizeof(int), c->stream));   // and kWaitFlag
     transform_locs_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(c->d_locs.p, c->d_tl.p, c->n, cc);
     LAUNCHED(c);
     double *linv = c->linv_slot(slot);
@@ -586,26 +607,26 @@ static bool residual_current(Ctx *c, const double *linv, const double *field, do
 static void ensure_logdet(Ctx *c) {
     if (c->logdet_valid) return;
     logdet_kernel<<<std::min(kReduceBlocks, (c->n + 255) / 256), 256, 0, c->stream>>>(
-        c->d_linv[c->cur].p, c->n, c->d_partials.p, reinterpret_cast<unsigned int *>(c->d_ticket.p + 1), c->d_logdet.p);
+        c->d_linv[c->cur].p, c->n, c->d_partials.p, reinterpret_cast<unsigned int *>(c->d_ticket.p + kCtaCount), c->d_logdet.p);
     LAUNCHED(c);
     c->logdet_valid = true;
 }
 
-// loglik_residual_kernel -> d_scalars[0..1]; spp: the kernel also closes the sweep it follows
+// loglik_residual_kernel -> pair A; spp: the kernel also closes the sweep it follows
 static void launch_loglik_residual(Ctx *c, const cudaLaunchConfig_t &lc, SweepParams *spp) {
     cudaLaunchConfig_t l = lc;
     l.gridDim = dim3(std::min(kReduceBlocks, (c->n + 255) / 256));
     l.blockDim = dim3(256);
     CK(cudaLaunchKernelEx(&l, loglik_residual_kernel, (const double *)c->d_r.p, c->n, (const double *)c->d_logdet.p, c->d_partials.p,
-                          reinterpret_cast<unsigned int *>(c->d_ticket.p + 1), spp, (unsigned long long)c->n_global, c->d_scalars.p));
+                          reinterpret_cast<unsigned int *>(c->d_ticket.p + kCtaCount), spp, (unsigned long long)c->n_global, c->d_scalars.p + kPairA));
 }
 
-// partial sums -> d_scalars[off..off+1].  allow_residual: the caller accepts the sums taken from the sweep's residual when
-// residual_current holds (they go to d_scalars[0..1], where the step graph writes them)
+// partial sums -> the pair of d_scalars at scal_off.  allow_residual: the caller accepts the sums taken from the sweep's residual when
+// residual_current holds (they go to pair A, where the step graph writes them)
 static void op_loglik_sums(Ctx *c, const double *linv, const double *field, double shift, int scal_off, bool allow_residual) {
     int blocks = std::min(kReduceBlocks, (c->n + 255) / 256);
     if (allow_residual && residual_current(c, linv, field, shift)) {
-        REQUIRE(scal_off == 0, "internal: the log-lik from the residual writes d_scalars[0..1], not [%d..%d]", scal_off, scal_off + 1);
+        REQUIRE(scal_off == kPairA, "internal: the log-lik from the residual writes pair A (d_scalars[%d]), not d_scalars[%d]", (int)kPairA, scal_off);
         ensure_logdet(c);
         cudaLaunchConfig_t lc = {};
         lc.stream = c->stream;
@@ -641,6 +662,29 @@ static const double *level_linv(Ctx *c, const double *linv) {
     return nullptr;
 }
 
+// The sync-free solve x = solve(linv, b) (and y = shift + scale * x) over `slots` rows of the padded row list `rows`.  Re-arms the
+// ticket and, if given, `arm` (x, or a sharded field's buffer of the next solve).  lv: the level-ordered copy of linv that goes with
+// d_rows_padded, or nullptr.  ss: the peers of a sharded solve, or nullptr.  A wait that times out sets kWaitFlag.
+static void launch_syncfree_solve(Ctx *c, const double *linv, const double *lv, const int *rows, int slots, const double *b,
+                                  unsigned long long *x, unsigned long long *arm, double *y, double shift, double scale,
+                                  const ShardSolve *ss) {
+    int *ticket = c->d_ticket.p + kSolveTicket, *err = c->d_nbad.p + kWaitFlag;
+    CK(cudaMemsetAsync(ticket, 0, sizeof(int), c->stream));
+    if (arm) {
+        fill_u64_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(arm, NNGP_SOLVE_SENTINEL, c->n);
+        LAUNCHED(c);
+    }
+    if (slots <= 0) return;
+    const int window = c->solve_window_ctas > 0 ? c->solve_window_ctas : c->n_sm * c->solve_ctas_per_sm;
+    const int blocks = std::max(1, std::min((slots + 255) / 256, window));
+    const unsigned int sleep_ns = (unsigned int)c->solve_sleep_ns;
+    if (ss && lv) { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT, true, true><<<blocks, 256, 0, c->stream>>>(c->d_nn_lvl.p, lv, rows, slots, b, x, y, shift, scale, slots, c->M, ticket, err, sleep_ns, *ss))); }
+    else if (ss) { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT, true><<<blocks, 256, 0, c->stream>>>(c->d_nn.p, linv, rows, slots, b, x, y, shift, scale, c->ld, c->M, ticket, err, sleep_ns, *ss))); }
+    else if (lv) { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT, false, true><<<blocks, 256, 0, c->stream>>>(c->d_nn_lvl.p, lv, rows, slots, b, x, y, shift, scale, slots, c->M, ticket, err, sleep_ns, ShardSolve{}, 0, c->solve_tl_on ? c->d_solve_tl.p : nullptr))); }
+    else { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT><<<blocks, 256, 0, c->stream>>>(c->d_nn.p, linv, rows, slots, b, x, y, shift, scale, c->ld, c->M, ticket, err, sleep_ns, ShardSolve{}))); }
+    LAUNCHED(c);
+}
+
 // x = solve(linv, b); optional y = shift + scale * x
 static void op_sptrsv(Ctx *c, const double *linv, const double *b, double *x, double *y, double shift, double scale) {
     if (c->sharded && c->world > 1) {
@@ -653,39 +697,17 @@ static void op_sptrsv(Ctx *c, const double *linv, const double *b, double *x, do
         const unsigned long long e = c->solve_epoch++;
         unsigned long long *xs = reinterpret_cast<unsigned long long *>(c->p2p_area + c->p2p_x_off + (size_t)(e & 1ull) * c->p2p_x_stride);
         unsigned long long *xs_next = reinterpret_cast<unsigned long long *>(c->p2p_area + c->p2p_x_off + (size_t)((e + 1ull) & 1ull) * c->p2p_x_stride);
-        CK(cudaMemsetAsync(c->d_ticket.p, 0, sizeof(int), c->stream));
-        fill_u64_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(xs_next, NNGP_SOLVE_SENTINEL, c->n);
-        LAUNCHED(c);
-        ShardSolve ss{};
-        ss.peers = c->peers;
-        ss.sxptr = c->d_sxptr.p;
-        ss.sxdst = c->d_sxdst.p;
+        ShardSolve ss{c->peers, c->d_sxptr.p, c->d_sxdst.p, {}};
         for (int h = 0; h < c->world; h++) ss.x_off[h] = c->peer_x_off[h] + (unsigned int)(e & 1ull) * c->peer_x_stride[h];
-        if (c->n_slots > 0) {
-            const int want = c->solve_window_ctas > 0 ? c->solve_window_ctas : c->n_sm * c->solve_ctas_per_sm;
-            const int blocks = std::max(1, std::min((c->n_slots + 255) / 256, want));
-            const double *lv = level_linv(c, linv);
-            if (lv) { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT, true, true><<<blocks, 256, 0, c->stream>>>(c->d_nn_lvl.p, lv, c->d_rows_padded.p, c->n_slots, b, xs, y, shift, scale, c->n_slots, c->M, c->d_ticket.p, c->d_nbad.p + 1, (unsigned int)c->solve_sleep_ns, ss))); }
-            else { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT, true><<<blocks, 256, 0, c->stream>>>(c->d_nn.p, linv, c->d_rows_padded.p, c->n_slots, b, xs, y, shift, scale, c->ld, c->M, c->d_ticket.p, c->d_nbad.p + 1, (unsigned int)c->solve_sleep_ns, ss))); }
-            LAUNCHED(c);
-        }
-        allreduce_scalars(c, 60, 1);   // barrier: every rank has finished this solve (and its stores into the peers' buffers)
+        launch_syncfree_solve(c, linv, level_linv(c, linv), c->d_rows_padded.p, c->n_slots, b, xs, xs_next, y, shift, scale, &ss);
+        allreduce_scalars(c, kBarrierSlot, 1);   // barrier: every rank has finished this solve (and its stores into the peers' buffers)
         shard_solve_ghosts_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(xs, c->d_owned.p, c->n, x, y, shift, scale);
         LAUNCHED(c);
         return;
     }
     if (c->solve_variant == 0) {
-        CK(cudaMemsetAsync(c->d_ticket.p, 0, sizeof(int), c->stream));
-        fill_u64_kernel<<<grid_for(c, c->n, 256), 256, 0, c->stream>>>(reinterpret_cast<unsigned long long *>(x), NNGP_SOLVE_SENTINEL, c->n);
-        LAUNCHED(c);
-        const int want = c->solve_window_ctas > 0 ? c->solve_window_ctas : c->n_sm * c->solve_ctas_per_sm;
-        const int blocks = std::max(1, std::min((c->n_slots + 255) / 256, want));
-        const double *lv = level_linv(c, linv);
-        const int slot0 = 0;
-        const int blocks_rest = std::max(1, std::min((c->n_slots - slot0 + 255) / 256, want));
-        if (lv) { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT, false, true><<<blocks_rest, 256, 0, c->stream>>>(c->d_nn_lvl.p, lv, c->d_rows_padded.p, c->n_slots, b, reinterpret_cast<unsigned long long *>(x), y, shift, scale, c->n_slots, c->M, c->d_ticket.p, c->d_nbad.p + 1, (unsigned int)c->solve_sleep_ns, ShardSolve{}, slot0, c->solve_tl_on ? c->d_solve_tl.p : nullptr))); }
-        else { DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT><<<blocks, 256, 0, c->stream>>>(c->d_nn.p, linv, c->d_rows_padded.p, c->n_slots, b, reinterpret_cast<unsigned long long *>(x), y, shift, scale, c->ld, c->M, c->d_ticket.p, c->d_nbad.p + 1, (unsigned int)c->solve_sleep_ns, ShardSolve{}))); }
-        LAUNCHED(c);
+        unsigned long long *xu = reinterpret_cast<unsigned long long *>(x);
+        launch_syncfree_solve(c, linv, level_linv(c, linv), c->d_rows_padded.p, c->n_slots, b, xu, xu, y, shift, scale, nullptr);
         return;
     }
     for (const auto &s : c->solve_plan) {
@@ -727,7 +749,7 @@ static ShardConst shard_const(Ctx *c) {
     sc.ginfo = c->d_ginfo.p;
     sc.tl = c->shard_tl_on ? c->d_shard_tl.p : nullptr;
     sc.state = c->d_shard_state.p;
-    sc.err = c->d_nbad.p + 1;
+    sc.err = c->d_nbad.p + kWaitFlag;
     sc.world = c->world; sc.rank = c->rank; sc.K = c->K;
     sc.val_off = (unsigned int)c->p2p_val_off;
     for (int h = 0; h < 8; h++) sc.peer_stride[h] = c->peer_stride[h];
@@ -853,7 +875,7 @@ static void op_sweeps(Ctx *c, int n_sweeps) {
     for (int s = 0; s < n_sweeps; s++) op_sweep(c, false);
 }
 
-// n_sweeps sweeps, then the log-lik sums of the current factor and the field at beta_0 = shift -> d_scalars[0..1].  Where the sums
+// n_sweeps sweeps, then the log-lik sums of the current factor and the field at beta_0 = shift -> pair A.  Where the sums
 // come from the sweep's residual, the last sweep is closed by the log-lik kernel itself (one chain of launches for the step); with
 // n_sweeps = 0 the log-lik is a launch of its own that leaves the sweep counter alone.
 static void op_sweeps_loglik(Ctx *c, int n_sweeps, double shift) {
@@ -864,11 +886,12 @@ static void op_sweeps_loglik(Ctx *c, int n_sweeps, double shift) {
         return;
     }
     op_sweeps(c, n_sweeps);
-    op_loglik_sums(c, c->d_linv[c->cur].p, c->d_field.p, shift, 0, true);
+    op_loglik_sums(c, c->d_linv[c->cur].p, c->d_field.p, shift, kPairA, true);
 }
 
 static void set_sweep_params(Ctx *c, double beta0, double log_scale, double log_noise_variance, int rng_mode, double seed) {
-    SweepParams *sp = reinterpret_cast<SweepParams *>(c->h_pinned + 32);
+    c->sweep_beta0 = beta0; c->sweep_log_scale = log_scale; c->sweep_log_noise_variance = log_noise_variance;
+    SweepParams *sp = &c->hs->sp;
     sp->beta0 = beta0;
     sp->e_ls = std::exp(-log_scale);
     sp->e_ln = std::exp(-log_noise_variance);
@@ -881,33 +904,45 @@ static void set_sweep_params(Ctx *c, double beta0, double log_scale, double log_
     CK(cudaMemcpyAsync(c->d_sp.p, sp, sizeof(SweepParams), cudaMemcpyHostToDevice, c->stream));
 }
 
-static void fetch_scalars(Ctx *c, int count) {
-    CK(cudaMemcpyAsync(c->h_pinned, c->d_scalars.p, sizeof(double) * count, cudaMemcpyDeviceToHost, c->stream));
+// pairs of d_scalars from pair A through last_pair -> hs->sums (at their slots); waits for the stream
+static const double *fetch_scalars(Ctx *c, int last_pair) {
+    CK(cudaMemcpyAsync(c->hs->sums, c->d_scalars.p + kPairA, sizeof(double) * (last_pair + 2 - kPairA), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
+    return c->hs->sums;
 }
 
-// the sync-free solve raises a device flag instead of spinning forever on a corrupted structure
-static void check_solve_flag(Ctx *c) {
-    int flag = 0;
-    CK(cudaMemcpyAsync(c->h_pinned + 9, c->d_nbad.p + 1, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+// a chain value every rank decides on: d_scalars[slot], just written, summed over the ranks -> pinned *host (after the next sync)
+static void allreduce_to_host(Ctx *c, int slot, double *host) {
+    allreduce_scalars(c, slot, 1);
+    CK(cudaMemcpyAsync(host, c->d_scalars.p + slot, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+}
+
+// The one reader of the device status, after all the stream holds: raises a wait that timed out (waits report one instead of spinning
+// forever on a corrupted structure or a dead peer), returns the rows whose block was not positive definite.  sum_ranks (the chain):
+// that count is summed over the ranks of a sharded field, so that every rank takes the same accept / reject decision.
+static int read_status(Ctx *c, bool sum_ranks = false) {
+    const bool reduce = sum_ranks && c->sharded && c->world > 1;
+    if (reduce) {
+        int_to_f64_kernel<<<1, 32, 0, c->stream>>>(c->d_nbad.p + kNotPd, c->d_scalars.p + kNotPdSlot);
+        LAUNCHED(c);
+        allreduce_to_host(c, kNotPdSlot, &c->hs->not_pd_sum);
+    }
+    const int *st = c->hs->status;
+    CK(cudaMemcpyAsync(c->hs->status, c->d_nbad.p, sizeof(c->hs->status), cudaMemcpyDeviceToHost, c->stream));
     CK(cudaStreamSynchronize(c->stream));
-    std::memcpy(&flag, c->h_pinned + 9, sizeof(int));
-    if (flag == 2) {
-        unsigned long long dbg[4] = {0, 0, 0, 0};
-        if (c->d_shard_state.p) cudaMemcpy(dbg, c->d_shard_state.p, sizeof(dbg), cudaMemcpyDeviceToHost);
-        int sdbg[3] = {0, 0, 0};
-        cudaMemcpy(sdbg, c->d_nbad.p + 3, sizeof(sdbg), cudaMemcpyDeviceToHost);
+    if (st[kWaitFlag] == 2) {
+        unsigned long long ss[kShardStateWords] = {};
+        if (c->d_shard_state.p) cudaMemcpy(ss, c->d_shard_state.p, sizeof(ss), cudaMemcpyDeviceToHost);
         set_error("sharded field: rank %d timed out waiting for a peer's halo value / reduction flag (a rank died or fell out of step); last halo wait recorded: colour %llu, ghost slot %llu, sweep %llu (this rank is at sweep %llu); last solve wait recorded: row %d for site %d in chunk %d",
-                  c->rank, dbg[1] + 1, dbg[2], dbg[3], dbg[0], sdbg[0], sdbg[1], sdbg[2]);
+                  c->rank, ss[kHaloWaitColour] + 1, ss[kHaloWaitSlot], ss[kHaloWaitSweep], ss[kSweepsSinceConnect], st[kSolveWaitRow], st[kSolveWaitSite], st[kSolveWaitChunk]);
         throw NcclFail();
     }
-    if (flag) {
-        int dbg[3] = {0, 0, 0};
-        cudaMemcpy(dbg, c->d_nbad.p + 3, sizeof(dbg), cudaMemcpyDeviceToHost);
+    if (st[kWaitFlag]) {
         set_error("triangular solve: dependency wait timed out (corrupted neighbour structure, or a peer of a sharded field that never delivered): rank %d, row (storage id) %d waited for site %d in chunk %d; owned = %d / %d",
-                  c->rank, dbg[0], dbg[1], dbg[2], c->sharded && c->d_owned.p ? 1 : 0, c->n);
+                  c->rank, st[kSolveWaitRow], st[kSolveWaitSite], st[kSolveWaitChunk], c->sharded && c->d_owned.p ? 1 : 0, c->n);
         throw CudaFail();
     }
+    return reduce ? (int)std::min(2.0e9, c->hs->not_pd_sum) : st[kNotPd];
 }
 
 static double ll_from_sums(Ctx *c, double sum_log, double sum_sq, double log_scale) {
@@ -935,7 +970,7 @@ static void op_beta0_sums(Ctx *c, int scal_off) {
 static void allreduce_scalars(Ctx *c, int off, int count) {
     if (c->sharded && c->world > 1 && c->p2p) {
         c->red_epoch++;
-        allreduce_p2p_kernel<<<1, 32, 0, c->stream>>>(c->peers, c->d_scalars.p + off, count, c->world, c->rank, c->p2p_slot_off, c->p2p_rflag_off, c->red_epoch, c->d_nbad.p + 1, c->d_scalars.p + off);
+        allreduce_p2p_kernel<<<1, 32, 0, c->stream>>>(c->peers, c->d_scalars.p + off, count, c->world, c->rank, c->p2p_slot_off, c->p2p_rflag_off, c->red_epoch, c->d_nbad.p + kWaitFlag, c->d_scalars.p + off);
         LAUNCHED(c);
         return;
     }
@@ -1000,11 +1035,8 @@ static void begin_sweeps(Ctx *c, double beta0, double log_scale, double log_nois
 }
 
 // nngp_time_op / nngp_time_op_group: Philox sweeps under a fixed seed with the scalar parameters of the context's last sweep
-// (set_sweep_params leaves them in h_pinned + 32)
 static void begin_timed_sweeps(Ctx *c) {
-    const SweepParams *sp = reinterpret_cast<SweepParams *>(c->h_pinned + 32);
-    begin_sweeps(c, sp->beta0, -std::log(sp->e_ls > 0 ? sp->e_ls : 1.0), -std::log(sp->e_ln > 0 ? sp->e_ln : 1.0), NNGP_RNG_PHILOX, nullptr, 1,
-                 12345.0);
+    begin_sweeps(c, c->sweep_beta0, c->sweep_log_scale, c->sweep_log_noise_variance, NNGP_RNG_PHILOX, nullptr, 1, 12345.0);
 }
 
 // ---- dense products with the resident design matrices (update_Gaussian.R:226-246) ----
@@ -1206,7 +1238,7 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
     CK(cudaEventCreateWithFlags(&c->ev_copy, cudaEventDisableTiming));
     CK(cudaEventCreate(&c->ev0));
     CK(cudaEventCreate(&c->ev1));
-    CK(cudaMallocHost(&c->h_pinned, 64 * sizeof(double)));
+    CK(cudaMallocHost(&c->hs, sizeof(HostScalars)));
 
     phase("cuda stream / events");
     // ---- validate structure, colour classes ----
@@ -1480,10 +1512,10 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
     c->d_lvl_ptr.upload(c->lvl_ptr, s); c->d_lm.upload(lm, s); c->d_optr.upload(optr, s); c->d_oidx.upload(oidx, s);
     c->d_cstart.upload(c->cstart, s); c->d_locs.upload(locs_int, s); c->d_nobs.upload(nobs, s);
     if (!c->partial_rows.empty()) c->d_partial_rows.upload(c->partial_rows, s);
-    c->d_nbad.alloc(8);   // [0] rows with a non-PD block, [1] wait timed out (1 solve, 2 halo / reduction), [3..5] which solve row waited for what
-    CK(cudaMemsetAsync(c->d_nbad.p, 0, 8 * sizeof(int), s));
-    c->d_ticket.alloc(2);   // [0] the triangular solve's chunk tickets, [1] last_cta_sum's CTA count (back to 0 after every launch)
-    CK(cudaMemsetAsync(c->d_ticket.p, 0, 2 * sizeof(int), s));
+    c->d_nbad.alloc(kStatusWords);
+    CK(cudaMemsetAsync(c->d_nbad.p, 0, kStatusWords * sizeof(int), s));
+    c->d_ticket.alloc(kTicketWords);
+    CK(cudaMemsetAsync(c->d_ticket.p, 0, kTicketWords * sizeof(int), s));
     c->d_rows_padded.upload(rows_padded, s);
     {   // level-ordered copies for the triangular solve: static neighbour table now, factor values at every factor build
         std::vector<int> lpos(n, -1), nn_lvl((size_t)c->n_slots * M, -1);
@@ -1509,7 +1541,7 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
     CK(cudaMemsetAsync(c->d_valT.p + c->nnz, 0, 2 * sizeof(double), s));
     c->d_pd.alloc(n); c->d_ymx.alloc(std::max(n_obs, 1)); c->d_S.alloc(n); c->d_field.alloc(n);
     c->d_newfield.alloc(n); c->d_r.alloc(n); c->d_tmp1.alloc(n); c->d_tmp2.alloc(n); c->d_io.alloc((size_t)std::max(n, n_obs));
-    c->d_zbuf.alloc(n); c->d_partials.alloc((size_t)kReduceBlocks * 4); c->d_scalars.alloc(64); c->d_logdet.alloc(1); c->d_sp.alloc(1);
+    c->d_zbuf.alloc(n); c->d_partials.alloc((size_t)kReduceBlocks * 4); c->d_scalars.alloc(kScalarSlots); c->d_logdet.alloc(1); c->d_sp.alloc(1);
     CK(cudaMemsetAsync(c->d_S.p, 0, sizeof(double) * n, s));
     if (sh) {
         const int W = sh->world;
@@ -1553,13 +1585,13 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
         CK(cudaMalloc(&c->p2p_area, c->p2p_doubles * sizeof(double)));
         CK(cudaMemsetAsync(c->p2p_area, 0, c->p2p_doubles * sizeof(double), s));
         {   // header: what a peer must know about this rank's area (read by the peers when they connect)
-            unsigned long long *hdr = reinterpret_cast<unsigned long long *>(c->h_pinned + 40);
+            unsigned long long *hdr = c->hs->area_hdr;
             hdr[0] = (unsigned long long)nrecv;
             hdr[1] = (unsigned long long)recv_proc.size();
             hdr[2] = (unsigned long long)c->p2p_x_off;
             hdr[3] = (unsigned long long)c->p2p_x_stride;
             hdr[4] = (unsigned long long)c->p2p_tab_off;
-            CK(cudaMemcpyAsync(c->p2p_area + c->p2p_hdr_off, hdr, 5 * sizeof(unsigned long long), cudaMemcpyHostToDevice, s));
+            CK(cudaMemcpyAsync(c->p2p_area + c->p2p_hdr_off, hdr, sizeof(c->hs->area_hdr), cudaMemcpyHostToDevice, s));
             c->recv_storage.resize(recv_proc.size());
             for (size_t k = 0; k < recv_proc.size(); k++) c->recv_storage[k] = psite[recv_proc[k]];
             if (!c->recv_storage.empty())
@@ -1567,8 +1599,8 @@ static void create_ctx_impl(const int *n_, const int *d_, const int *m_, const d
         }
         c->d_recvbuf = c->p2p_area + c->p2p_val_off;
         ensure_stage(c, (size_t)std::max(n, n_obs));   // no page-locked allocation (a device-synchronising call) once peers may be waiting on this rank
-        c->d_shard_state.alloc(4);
-        CK(cudaMemsetAsync(c->d_shard_state.p, 0, 4 * sizeof(unsigned long long), s));
+        c->d_shard_state.alloc(kShardStateWords);
+        CK(cudaMemsetAsync(c->d_shard_state.p, 0, kShardStateWords * sizeof(unsigned long long), s));
         CK(cudaStreamSynchronize(s));
         if (W > 1 && sh->comm_id[0] != '\0') {   // collective: every rank of the field creates its context at the same time
             nccl_load();
@@ -1676,7 +1708,7 @@ void nngp_shard_timeline(const int *ctx_id, const double *beta_0, const double *
     unsigned long long t0 = ~0ull;
     for (size_t i = 0; i < cnt; i++) if (t[i] != 0ull && t[i] != ~0ull && t[i] < t0) t0 = t[i];
     for (size_t i = 0; i < cnt; i++) out_ns[i] = (t[i] == 0ull || t[i] == ~0ull) ? -1.0 : (double)(t[i] - t0);
-    check_solve_flag(c);
+    read_status(c);
     ABI_END
 }
 
@@ -1689,8 +1721,7 @@ void nngp_solve_timeline(const int *ctx_id, double *out_ns, int *level_of_chunk,
     REQUIRE(out_ns && level_of_chunk && n_chunks, "nngp_solve_timeline: null argument");
     NEED(!c->sharded && c->have_slot(NNGP_SLOT_CURRENT) && c->have_field, "nngp_solve_timeline: needs an unsharded context with a factor and a field");
     use(c);
-    const int slot0 = 0;
-    const int nc = (c->n_slots - slot0 + 255) / 256;
+    const int nc = (c->n_slots + 255) / 256;
     REQUIRE(*n_chunks >= nc, "nngp_solve_timeline: need room for %d chunks", nc);
     c->d_solve_tl.alloc((size_t)nc + 1);
     CK(cudaMemsetAsync(c->d_solve_tl.p, 0, sizeof(unsigned long long) * ((size_t)nc + 1), c->stream));
@@ -1706,7 +1737,7 @@ void nngp_solve_timeline(const int *ctx_id, double *out_ns, int *level_of_chunk,
     // level of a slot: levels are padded to warps, so walk the padded level starts
     std::vector<int> slot_level((size_t)c->n_slots, 0);
     { int tpos = 0; for (int l = 0; l < c->n_levels; l++) { const int w = c->lvl_ptr[l + 1] - c->lvl_ptr[l]; const int wp = (w + 31) / 32 * 32; for (int u = 0; u < wp && tpos < c->n_slots; u++) slot_level[tpos++] = l; } }
-    for (int k = 0; k < nc; k++) { out_ns[k] = t[k] ? (double)(t[k] - t0) : -1.0; level_of_chunk[k] = slot_level[(size_t)slot0 + (size_t)k * 256]; }
+    for (int k = 0; k < nc; k++) { out_ns[k] = t[k] ? (double)(t[k] - t0) : -1.0; level_of_chunk[k] = slot_level[(size_t)k * 256]; }
     *n_chunks = nc;
     ABI_END
 }
@@ -1728,10 +1759,7 @@ void nngp_factor_build(const int *ctx_id, const int *slot, const double *covparm
     const CovConst cc = make_cov(c, covparms, *n_covparms);
     c->last_cc = cc; c->have_cc = true;
     op_factor_build(c, *slot, cc);
-    int bad = 0;
-    CK(cudaMemcpyAsync(c->h_pinned, c->d_nbad.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-    CK(cudaStreamSynchronize(c->stream));
-    std::memcpy(&bad, c->h_pinned, sizeof(int));
+    const int bad = read_status(c);
     if (n_not_pd) *n_not_pd = bad;
     ABI_END
 }
@@ -1830,9 +1858,9 @@ void nngp_loglik(const int *ctx_id, const int *slot, const double *beta_0, const
     NEED(c->have_slot(*slot), "nngp_loglik: that slot holds no factor");
     NEED(c->have_field, "nngp_loglik: no field on the device");
     use(c);
-    op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, 0, true);
-    fetch_scalars(c, 2);
-    *ll = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], *log_scale);
+    op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, kPairA, true);
+    const double *s = fetch_scalars(c, kPairA);
+    *ll = ll_from_sums(c, s[0], s[1], *log_scale);
     ABI_END
 }
 
@@ -1843,9 +1871,9 @@ void nngp_loglik_host(const int *ctx_id, const int *slot, const double *z, const
     NEED(c->have_slot(*slot), "nngp_loglik_host: that slot holds no factor");
     use(c);
     upload_site_vector(c, z, c->d_tmp1.p);
-    op_loglik_sums(c, c->linv_slot(*slot), c->d_tmp1.p, 0.0, 0, false);
-    fetch_scalars(c, 2);
-    *ll = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], *log_scale);
+    op_loglik_sums(c, c->linv_slot(*slot), c->d_tmp1.p, 0.0, kPairA, false);
+    const double *s = fetch_scalars(c, kPairA);
+    *ll = ll_from_sums(c, s[0], s[1], *log_scale);
     ABI_END
 }
 
@@ -1885,7 +1913,7 @@ void nngp_sptrsv(const int *ctx_id, const int *slot, const double *b, double *x,
     op_sptrsv(c, c->linv_slot(*slot), c->d_tmp1.p, c->d_tmp2.p, nullptr, 0.0, 1.0);
     CK(cudaGetLastError());
     download_site_vector(c, c->d_tmp2.p, x);
-    check_solve_flag(c);
+    read_status(c);
     ABI_END
 }
 
@@ -1902,7 +1930,7 @@ void nngp_gibbs_sweep(const int *ctx_id, const int *n_sweeps, const double *beta
     begin_sweeps(c, *beta_0, *log_scale, *log_noise_variance, *rng_mode, z, *n_sweeps, seed ? *seed : 0.0);
     op_sweeps(c, *n_sweeps);
     CK(cudaStreamSynchronize(c->stream));
-    if (c->p2p) check_solve_flag(c);
+    if (c->p2p) read_status(c);
     ABI_END
 }
 
@@ -1938,17 +1966,16 @@ void nngp_sweep_loglik_host(const int *ctx_id, const int *n_sweeps, const double
         CK(cudaEventRecord(c->ev_copy, c->stream));
         CK(cudaStreamWaitEvent(c->copy_stream, c->ev_copy, 0));
         CK(cudaMemcpyAsync(field_io, c->d_io.p, sizeof(double) * c->n, cudaMemcpyDeviceToHost, c->copy_stream));
-        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, 0, true);
-        CK(cudaMemcpyAsync(c->h_pinned, c->d_scalars.p, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
+        op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, kPairA, true);
+        fetch_scalars(c, kPairA);
         CK(cudaStreamSynchronize(c->copy_stream));
     } else {
         op_sweeps_loglik(c, *n_sweeps, *beta_0);
-        CK(cudaMemcpyAsync(c->h_pinned, c->d_scalars.p, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
+        CK(cudaMemcpyAsync(c->hs->sums, c->d_scalars.p + kPairA, sizeof(double) * 2, cudaMemcpyDeviceToHost, c->stream));
         download_site_vector(c, c->d_field.p, field_io);   // synchronises
     }
-    *ll = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], *log_scale);
-    if (c->p2p) check_solve_flag(c);
+    *ll = ll_from_sums(c, c->hs->sums[kPairA], c->hs->sums[kPairA + 1], *log_scale);
+    if (c->p2p) read_status(c);
     ABI_END
 }
 
@@ -2012,7 +2039,7 @@ static void finish_p2p_connect(Ctx *c, const int *peer_recv_base) {
         }
     c->d_bptr.upload(bptr, c->stream);
     c->d_bdst.upload(bdst, c->stream);
-    CK(cudaMemsetAsync(c->d_shard_state.p, 0, 4 * sizeof(unsigned long long), c->stream));
+    CK(cudaMemsetAsync(c->d_shard_state.p, 0, kShardStateWords * sizeof(unsigned long long), c->stream));
     // every ghost slot (both parities) starts EMPTY: the value itself is the message (see NNGP_HALO_EMPTY)
     fill_u64_kernel<<<grid_for(c, (long long)(2 * c->p2p_parity_stride), 256), 256, 0, c->stream>>>(reinterpret_cast<unsigned long long *>(c->p2p_area + c->p2p_val_off), NNGP_HALO_EMPTY, (int)(2 * c->p2p_parity_stride));
     CK(cudaStreamSynchronize(c->stream));
@@ -2101,7 +2128,7 @@ void nngp_shard_group_sweep(const int *ctx_ids, const int *world, const int *n_s
     for (int s = 0; s < *n_sweeps; s++)       // sweep by sweep over the members: no stream runs far ahead of its peers
         for (Ctx *c : cs) { use(c); op_sweeps(c, 1); }
     for (Ctx *c : cs) { use(c); CK(cudaStreamSynchronize(c->stream)); }
-    for (Ctx *c : cs) { use(c); check_solve_flag(c); }
+    for (Ctx *c : cs) { use(c); read_status(c); }
     ABI_END
 }
 
@@ -2117,14 +2144,14 @@ void nngp_shard_group_loglik(const int *ctx_ids, const int *world, const int *sl
         NEED(cs[h]->sharded && (cs[h]->p2p || W == 1), "nngp_shard_group_loglik: the contexts are not connected (nngp_shard_connect_local)");
         NEED(cs[h]->have_slot(*slot) && cs[h]->have_field, "nngp_shard_group_loglik: factor and field must be set first");
     }
-    for (Ctx *c : cs) { use(c); op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, 0, false); }
+    for (Ctx *c : cs) { use(c); op_loglik_sums(c, c->linv_slot(*slot), c->d_field.p, *beta_0, kPairA, false); }
     for (int h = 0; h < W; h++) {
         Ctx *c = cs[h];
         use(c);
-        fetch_scalars(c, 2);
-        ll[h] = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], *log_scale);
+        const double *s = fetch_scalars(c, kPairA);
+        ll[h] = ll_from_sums(c, s[0], s[1], *log_scale);
     }
-    for (Ctx *c : cs) { use(c); check_solve_flag(c); }
+    for (Ctx *c : cs) { use(c); read_status(c); }
     ABI_END
 }
 
@@ -2218,12 +2245,12 @@ void nngp_ancillary_propose(const int *ctx_id, const double *beta_0, const doubl
     // tmp1 = current %*% (field - beta_0); tmp2 = solve(proposal, tmp1); newfield = beta_0 + exp(.5 dls) * tmp2
     op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, *beta_0, c->d_tmp1.p);
     op_sptrsv(c, c->linv_slot(NNGP_SLOT_PROPOSAL), c->d_tmp1.p, c->d_tmp2.p, c->d_newfield.p, *beta_0, std::exp(0.5 * *delta_log_scale));
-    op_obs_sq(c, c->d_newfield.p, c->d_field.p, 0);
+    op_obs_sq(c, c->d_newfield.p, c->d_field.p, kPairA);
     CK(cudaGetLastError());
-    fetch_scalars(c, 2);
-    check_solve_flag(c);
+    const double *s = fetch_scalars(c, kPairA);
+    read_status(c);
     // sum(dnorm(y, new) - dnorm(y, old)) = -(SSR_new - SSR_old) / (2 tau^2)
-    *field_response_ratio = -0.5 * (c->h_pinned[0] - c->h_pinned[1]) * std::exp(-*log_noise_variance);
+    *field_response_ratio = -0.5 * (s[0] - s[1]) * std::exp(-*log_noise_variance);
     c->have_newfield = true;
     ABI_END
 }
@@ -2247,9 +2274,9 @@ void nngp_beta0_moments(const int *ctx_id, const double *log_scale, double *mean
     REQUIRE(log_scale && mean && var, "nngp_beta0_moments: bad argument");
     NEED(c->have_slot(NNGP_SLOT_CURRENT) && c->have_field, "nngp_beta0_moments: needs a current factor and a field");
     use(c);
-    op_beta0_sums(c, 0);
-    fetch_scalars(c, 2);
-    const double vv = c->h_pinned[0], uv = c->h_pinned[1];
+    op_beta0_sums(c, kPairA);
+    const double *s = fetch_scalars(c, kPairA);
+    const double vv = s[0], uv = s[1];
     *var = (1.0 / vv) * std::exp(*log_scale);
     *mean = std::exp(-*log_scale) * uv * *var;
     ABI_END
@@ -2261,9 +2288,8 @@ void nngp_ssr(const int *ctx_id, double *ssr, int *status) {
     REQUIRE(ssr != nullptr, "null ssr");
     NEED(c->have_field && c->have_obs, "nngp_ssr: field and observations must be set first");
     use(c);
-    op_obs_sq(c, c->d_field.p, c->d_field.p, 0);
-    fetch_scalars(c, 2);
-    *ssr = c->h_pinned[0];
+    op_obs_sq(c, c->d_field.p, c->d_field.p, kPairA);
+    *ssr = fetch_scalars(c, kPairA)[0];
     ABI_END
 }
 
@@ -2276,7 +2302,7 @@ void nngp_field_init(const int *ctx_id, const int *slot, const double *beta_0, c
     upload_site_vector(c, z, c->d_tmp1.p);
     op_sptrsv(c, c->linv_slot(*slot), c->d_tmp1.p, c->d_tmp2.p, c->d_field.p, *beta_0, std::sqrt(std::exp(*log_scale)));
     CK(cudaGetLastError());
-    check_solve_flag(c);
+    read_status(c);
     c->have_field = true;
     ABI_END
 }
@@ -2326,17 +2352,11 @@ void nngp_predict_sample(const int *ctx_id, const int *slot, const int *n_obs_si
     upload_site_vector(c, host.data(), c->d_tmp1.p);     // known x on the observed rows, rhs z on the new rows
     predict_prepare_kernel<<<grid_for(c, n, 256), 256, 0, c->stream>>>(reinterpret_cast<unsigned long long *>(c->d_tmp2.p), c->d_tmp1.p, c->d_i2g.p, n0, n);
     LAUNCHED(c);
-    if (c->pred_slots > 0) {
-        CK(cudaMemsetAsync(c->d_ticket.p, 0, sizeof(int), c->stream));
-        const int want = c->solve_window_ctas > 0 ? c->solve_window_ctas : c->n_sm * c->solve_ctas_per_sm;
-        const int blocks = std::max(1, std::min((c->pred_slots + 255) / 256, want));
-        const double *linv = c->linv_slot(*slot);
-        DISPATCH_MT(c->M, (sptrsv_syncfree_kernel<MT><<<blocks, 256, 0, c->stream>>>(c->d_nn.p, linv, c->d_pred_rows.p, c->pred_slots, c->d_tmp1.p, reinterpret_cast<unsigned long long *>(c->d_tmp2.p), nullptr, 0.0, 1.0, c->ld, c->M, c->d_ticket.p, c->d_nbad.p + 1, (unsigned int)c->solve_sleep_ns, ShardSolve{})));
-        LAUNCHED(c);
-    }
+    launch_syncfree_solve(c, c->linv_slot(*slot), nullptr, c->d_pred_rows.p, c->pred_slots, c->d_tmp1.p,   // x is armed: prepared above
+                          reinterpret_cast<unsigned long long *>(c->d_tmp2.p), nullptr, nullptr, 0.0, 1.0, nullptr);
     CK(cudaGetLastError());
     download_site_vector(c, c->d_tmp2.p, host.data());
-    check_solve_flag(c);
+    read_status(c);
     for (int i = 0; i < np; i++) out[i] = sd * host[n0 + i];
     ABI_END
 }
@@ -2398,16 +2418,13 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
     // a sharded field: every rank runs this loop on its block with the same scalar state and the same R stream; all scalars
     // that enter a decision are all-reduced (rank-ordered sums, identical everywhere), so the ranks stay in step
     if (c->n_obs_global < 0) {
+        c->hs->n_obs_sum = (double)c->n_obs;
         if (c->sharded && c->world > 1) {
-            c->h_pinned[16] = (double)c->n_obs;
-            CK(cudaMemcpyAsync(c->d_scalars.p + 16, c->h_pinned + 16, sizeof(double), cudaMemcpyHostToDevice, c->stream));
-            allreduce_scalars(c, 16, 1);
-            CK(cudaMemcpyAsync(c->h_pinned + 16, c->d_scalars.p + 16, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+            CK(cudaMemcpyAsync(c->d_scalars.p + kNObsSlot, &c->hs->n_obs_sum, sizeof(double), cudaMemcpyHostToDevice, c->stream));
+            allreduce_to_host(c, kNObsSlot, &c->hs->n_obs_sum);
             CK(cudaStreamSynchronize(c->stream));
-            c->n_obs_global = c->h_pinned[16];
-        } else {
-            c->n_obs_global = (double)c->n_obs;
         }
+        c->n_obs_global = c->hs->n_obs_sum;
     }
     const double n_obs = c->n_obs_global;
     const int n_obs_local = c->n_obs;
@@ -2419,23 +2436,6 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         for (int j = 0; j < ns; j++) cp[1 + j] = (matern && j == ns - 1) ? 0.5 + 0.5 / (1.0 + std::exp(-sh[j])) : std::exp(sh[j]);
         cp[1 + ns] = 0.0;
         return make_cov(c, cp, ns + 2);
-    };
-    auto n_bad = [&]() {   // rows whose block was not positive definite; also surfaces a solve / halo wait that timed out
-        int bad[2];
-        const bool reduce = c->sharded && c->world > 1;
-        if (reduce) {   // the accept / reject decision must be the same on every rank: sum the counts over the ranks
-            int_to_f64_kernel<<<1, 32, 0, c->stream>>>(c->d_nbad.p, c->d_scalars.p + 17);
-            LAUNCHED(c);
-            allreduce_scalars(c, 17, 1);
-            CK(cudaMemcpyAsync(c->h_pinned + 17, c->d_scalars.p + 17, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-        }
-        CK(cudaMemcpyAsync(c->h_pinned + 8, c->d_nbad.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
-        CK(cudaStreamSynchronize(c->stream));
-        std::memcpy(bad, c->h_pinned + 8, 2 * sizeof(int));
-        if (reduce) bad[0] = (int)std::min(2.0e9, c->h_pinned[17]);
-        if (bad[1] == 2) { set_error("sharded field: timed out waiting for a peer's halo / reduction flag (a rank died or fell out of step)"); throw NcclFail(); }
-        if (bad[1]) { set_error("triangular solve: dependency wait timed out (corrupted neighbour structure?)"); throw CudaFail(); }
-        return bad[0];
     };
     RStream rs;
     rs.set_seed((uint32_t)(iter_start + *chain_index_));                         // :36
@@ -2475,10 +2475,10 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         op_factor_build(c, NNGP_SLOT_PROPOSAL, to_covparms(new_shape));          // :123
         op_spmv(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, beta_0, c->d_tmp1.p);
         op_sptrsv(c, c->linv_slot(NNGP_SLOT_PROPOSAL), c->d_tmp1.p, c->d_tmp2.p, c->d_newfield.p, beta_0, std::exp(.5 * (new_log_scale - log_scale)));  // :127
-        op_obs_sq(c, c->d_newfield.p, c->d_field.p, 0);
-        fetch_scalars(c, 2);
-        const int bad_a = n_bad();
-        const double ratio = -0.5 * (c->h_pinned[0] - c->h_pinned[1]) * std::exp(-lnv);   // :129-131
+        op_obs_sq(c, c->d_newfield.p, c->d_field.p, kPairA);
+        const double *obs_sq = fetch_scalars(c, kPairA);
+        const int bad_a = read_status(c, true);
+        const double ratio = -0.5 * (obs_sq[0] - obs_sq[1]) * std::exp(-lnv);    // :129-131
         if (ratio + 0.0 > std::log(rs.unif_rand()) && bad_a == 0) {              // :133
             std::memcpy(shape, new_shape, sizeof(double) * ns);
             log_scale = new_log_scale;
@@ -2505,12 +2505,12 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         if (std::exp(new_log_scale) < var_y) {                                    // :167
             for (int k = 0; k < ns; k++) new_shape[k] = shape[k] + innovation[1 + k];
             op_factor_build(c, NNGP_SLOT_PROPOSAL, to_covparms(new_shape));      // :179
-            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_PROPOSAL), c->d_field.p, beta_0, 0, false);
-            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, beta_0, 2, false);
-            fetch_scalars(c, 4);
-            const int bad_s = n_bad();
-            const double GP_ratio = ll_from_sums(c, c->h_pinned[0], c->h_pinned[1], new_log_scale) -
-                                    ll_from_sums(c, c->h_pinned[2], c->h_pinned[3], log_scale);   // :184-186
+            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_PROPOSAL), c->d_field.p, beta_0, kPairA, false);
+            op_loglik_sums(c, c->linv_slot(NNGP_SLOT_CURRENT), c->d_field.p, beta_0, kPairB, false);
+            const double *ll_sums = fetch_scalars(c, kPairB);
+            const int bad_s = read_status(c, true);
+            const double GP_ratio = ll_from_sums(c, ll_sums[kPairA], ll_sums[kPairA + 1], new_log_scale) -
+                                    ll_from_sums(c, ll_sums[kPairB], ll_sums[kPairB + 1], log_scale);   // :184-186
             if (GP_ratio > std::log(rs.unif_rand()) && bad_s == 0) {              // :189
                 std::memcpy(shape, new_shape, sizeof(double) * ns);
                 log_scale = new_log_scale;
@@ -2532,10 +2532,10 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         // ---- (C) beta_0 :219-224 (no location-level regressors) ----
         nvtxRangePushA("nngp C mean parameters");
         if (reg_q == 0) {
-            op_beta0_sums(c, 0);
-            fetch_scalars(c, 2);
-            const double bvar = (1.0 / c->h_pinned[0]) * std::exp(log_scale);
-            const double b0mean = std::exp(-log_scale) * c->h_pinned[1] * bvar;
+            op_beta0_sums(c, kPairA);
+            const double *b0_sums = fetch_scalars(c, kPairA);
+            const double bvar = (1.0 / b0_sums[0]) * std::exp(log_scale);
+            const double b0mean = std::exp(-log_scale) * b0_sums[1] * bvar;
             beta_0 = b0mean + std::sqrt(bvar) * rs.norm_rand();
         }
         // ---- (C') regression coefficients :226-250 ----
@@ -2603,9 +2603,8 @@ static void chain_run_impl(Ctx *c, const int *n_shape_, double *params_io, const
         nvtxRangePop();
         // ---- (E) noise variance :281-293 ----
         nvtxRangePushA("nngp E noise variance");
-        op_obs_sq(c, c->d_field.p, c->d_field.p, 0);
-        fetch_scalars(c, 2);
-        const double ssr = c->h_pinned[0];
+        op_obs_sq(c, c->d_field.p, c->d_field.p, kPairA);
+        const double ssr = fetch_scalars(c, kPairA)[0];
         for (int k = 0; k < 10; k++) {
             const double inn = 0.0 + .01 * rs.norm_rand();
             if (std::exp(lnv + inn) < var_y) {
